@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the hot path (BASELINE.json): Mrays/s (primary + secondary).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config C1|C2|C3|C5] [--no-extras]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config C1|C2|C3|C5] [--no-extras] [--dump-outputs DIR]
 
 Default workload = BASELINE config C2: procedural ~1M-triangle displaced mesh in an emitter-lit room, 1920x1080, 1 spp per pass,
 depth 8 (bounces = 6), GGX + diffuse.  A step = one progressive pass over the whole frame.  N>1 (torchrun, one rank per GPU): the scene
@@ -18,6 +18,13 @@ One JSON line on rank 0:
   parity       the GPU accumulation of one sample bit-compared with the oracle image of that cpu_baseline sample, plus hit ids
   configs      (N=1, default config) compact runs of the other BASELINE configs C1, C3, C5 with their own roofline + parity
   c4_strong    BASELINE config C4 (4K progressive render split by samples over the N GPUs, one reduce per pass): strong scaling
+`--dump-outputs DIR` writes, after the timed steps, what the timed path computed in its last step, at most 64 MB in all: for a render
+config accum.npy (gPermanentData, H x W x 4 float32; above 2^21 pixels, as C3's 3840x2160, a fixed, seeded sample of pixels, n x 4,
+with their row-major indices in accum_rows.npy) and counters.npy (closest rays, shadow rays, paths of the timed steps); for C5 the hit
+records (t, u, v, prim, inst as float64) of a fixed, seeded sample of each batch, with the sampled rows.  The inputs are seeded: two
+builds run with the same arguments can be compared array by array.  Except C5's incoherent batch: its rays start at the coherent
+batch's hit points and only rays that hit are kept, so a build whose coherent t differs in any bit traces other incoherent rays, and
+its sampled rows are drawn from a batch of another size; compare hits_incoherent row by row only where hits_coherent agree exactly.
 `--impl reference` times the CPU port on all host threads (the reference itself is a Windows/DX12 application and cannot run); it loads
 no engine library and prints the same `config`.
 """
@@ -55,7 +62,39 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the compact runs of the other BASELINE configs and C4")
     ap.add_argument("--c4-spp", type=int, default=16, help="samples per pixel of one C4 step (split over the ranks)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the timed path computed in its last step as DIR/<name>.npy (rank 0)")
     return ap.parse_args()
+
+
+DUMP_MAX_BYTES = 64 * 10 ** 6      # everything --dump-outputs writes in one run
+DUMP_SAMPLE_PIXELS = 1 << 21       # accumulation pixels kept when the whole buffer would not fit (32 MB float32 + 16 MB indices)
+DUMP_SAMPLE_RAYS = 1 << 19         # hit records kept per C5 batch (2 x (20 MB float64 + 4 MB indices))
+_dumped_bytes = 0
+
+
+def dump_outputs(d, arrays):
+    """Writes {name: array} as d/<name>.npy in float32 or float64, so that two builds can be compared output by output."""
+    global _dumped_bytes
+    arrays = {name: np.asarray(a) for name, a in arrays.items()}
+    arrays = {name: a if a.dtype in (np.float32, np.float64) else a.astype(np.float64) for name, a in arrays.items()}
+    _dumped_bytes += sum(a.nbytes for a in arrays.values())
+    if _dumped_bytes > DUMP_MAX_BYTES:
+        raise SystemExit("bench.py: --dump-outputs would write %d bytes, more than %d" % (_dumped_bytes, DUMP_MAX_BYTES))
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
+def seeded_rows(n, k):
+    """A fixed sample of k of n row indices (all of them when k >= n), in ascending order."""
+    return np.arange(n) if k >= n else np.sort(np.random.RandomState(0).choice(n, k, replace=False))
+
+
+def hit_records(h):
+    """rtx_trace_device's 5-word hit records (t, u, v as float32; prim, inst as uint32) as float64 columns."""
+    h = np.ascontiguousarray(h, dtype=np.float32)
+    return np.concatenate([h[:, :3].astype(np.float64), h[:, 3:].view(np.uint32).astype(np.float64)], axis=1)
 
 
 # ------------------------------------------------------------------------------------------------ workloads (BASELINE.json configs)
@@ -463,6 +502,17 @@ def run_render(rtdx, D, cfg, args, steps, warmup, full):
     ms = e0.elapsed_time(e1)
     clk = clocks.stop() if clocks else None
     cnt = ctx.counters()
+    if full and args.dump_outputs and rank == 0:
+        # gPermanentData after the last timed pass (the sum of the warm-up and timed samples; with N ranks, the reduced sum) and the
+        # ray / path counts of the timed steps, before the roofline and e2e legs render into the same context
+        accum = ctx.read_accum().reshape(-1, 4)
+        out = {"counters": [cnt["closest_rays"], cnt["shadow_rays"], cnt["paths"]]}
+        if accum.shape[0] > DUMP_SAMPLE_PIXELS:
+            out["accum_rows"] = seeded_rows(accum.shape[0], DUMP_SAMPLE_PIXELS)
+            out["accum"] = accum[out["accum_rows"]]
+        else:
+            out["accum"] = accum.reshape(H, W, 4)
+        dump_outputs(args.dump_outputs, out)
     rays = cnt["closest_rays"] + cnt["shadow_rays"]
     mx, sm = D.max_sum([ms, float(rays), float(cnt["kernel_launches"])])
     ms, rays_all, launches = mx[0], sm[1], int(sm[2])
@@ -574,6 +624,10 @@ def run_trace(rtdx, D, cfg, args, steps, warmup):
             ctx.trace_device(r.data_ptr(), m, h.data_ptr())
         e1.record(); torch.cuda.synchronize()
         ms = e0.elapsed_time(e1) / steps
+        if args.dump_outputs and D.rank == 0:
+            keep = seeded_rows(m, DUMP_SAMPLE_RAYS)
+            dump_outputs(args.dump_outputs, {"hits_" + name: hit_records(h[torch.from_numpy(keep).cuda()].cpu().numpy()),
+                                             "hits_%s_rows" % name: keep})
         out[name] = {"rays": int(m), "ms_per_batch": ms, "value": m / ms / 1e3, "bytes_per_ray": b_ray, "achieved_gbs": m * b_ray / ms / 1e6,
                      "frac": m * b_ray / ms / 1e6 / peak, "nodes_per_ray": st["nodes_visited"] / m, "tris_per_ray": st["tris_tested"] / m}
     total_rays = out["coherent"]["rays"] + out["incoherent"]["rays"]
@@ -656,6 +710,7 @@ def main():
                 extras[name] = {k: r.get(k) for k in ("config", "value", "ms_per_step", "rays_per_path", "roofline", "cpu_baseline", "parity")}
             for tris in (1_000_000, 10_000_000):
                 a2 = argparse.Namespace(**vars(args)); a2.tris = tris; a2.no_cpu_baseline = args.no_cpu_baseline or tris > 2_000_000
+                a2.dump_outputs = ""
                 r = run_trace(rtdx, D, config_of("C5", a2), a2, 5, 2)
                 extras["C5_%dM" % (tris // 1_000_000)] = {k: r.get(k) for k in ("config", "value", "ms_per_step", "batches", "roofline", "cpu_baseline", "parity", "blas")}
         c4 = run_c4_strong(rtdx, D, args)
