@@ -77,6 +77,7 @@ typedef struct {
     uint64_t closest_rays, shadow_rays, paths;   /* TraceRay-equivalents actually issued since the last reset */
     uint64_t kernel_launches;                    /* launches of this library's own kernels */
     uint64_t nodes_visited, tris_tested, instances_entered;   /* only counted by rtx_trace_stats */
+    uint64_t shading_replays;    /* paths the shading stages re-ran with guarded IEEE operations (RTX_OPT_TRACE_STATS only) */
 } rtx_counters;
 
 typedef struct {
@@ -171,7 +172,8 @@ rtx_status rtx_last_pass_ms(rtx_ctx*, float* trace_ms, float* total_ms);
 #define RTX_STAGE_COUNT 10
 rtx_status rtx_last_pass_stage_ms(rtx_ctx*, float* ms_by_stage, uint32_t n_stages, float* total_ms);
 /* runtime options.  RTX_OPT_TRACE_STATS: closest-hit traversals of rtx_render_pass also count nodes/triangles/instances
- * (instrumented kernel variant: for the roofline's B_ray, never for timed runs).  RTX_OPT_STAGE_TIMING: record CUDA events
+ * (instrumented kernel variant: for the roofline's B_ray, never for timed runs), and the shading stages count the paths they
+ * replay with guarded IEEE operations (rtx_counters.shading_replays).  RTX_OPT_STAGE_TIMING: record CUDA events
  * around every traversal launch of a pass so that rtx_last_pass_ms can report the traversal share.
  * RTX_OPT_PASS_PARTS: 1..4 path ranges of a pass that run concurrently on separate CUDA streams (default 2; the image
  * does not depend on it; passes with per-launch events, statistics or ReSTIR reuse always run as one part). */
@@ -196,7 +198,8 @@ rtx_status rtx_set_option(rtx_ctx*, uint32_t option, uint32_t value);
 /* debug: per-pixel record of one sample in the layout of the oracle's orc_debug_pixel (64 floats) */
 rtx_status rtx_debug_pixel(rtx_ctx*, uint32_t x, uint32_t y, float* out64);
 /* self-test of the device arithmetic (csrc/dmath.cuh): compares every hand-scheduled fast path with the IEEE-754
- * operation it restates over ALL 2^32 binary32 bit patterns on the device.  mismatches_out[0] = d_rsqrt vs 1/sqrt. */
+ * operation it restates over ALL 2^32 binary32 bit patterns on the device.  mismatches_out[0] = d_rsqrt vs 1/sqrt; [2..6] = the
+ * unguarded fast paths (result or range flag wrong): sqrt, rcp, rsqrt, a/b on 2^34 pairs, a/3 and a/pi on every a. */
 rtx_status rtx_selftest_dmath(rtx_ctx*, uint64_t* mismatches_out, uint32_t n_out);
 
 #ifdef __cplusplus

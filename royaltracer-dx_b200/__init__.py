@@ -48,7 +48,8 @@ class RtxConfig(C.Structure):
 
 class RtxCounters(C.Structure):
     _fields_ = [("closest_rays", C.c_uint64), ("shadow_rays", C.c_uint64), ("paths", C.c_uint64), ("kernel_launches", C.c_uint64),
-                ("nodes_visited", C.c_uint64), ("tris_tested", C.c_uint64), ("instances_entered", C.c_uint64)]
+                ("nodes_visited", C.c_uint64), ("tris_tested", C.c_uint64), ("instances_entered", C.c_uint64),
+                ("shading_replays", C.c_uint64)]
 
 
 class RtxBlasInfo(C.Structure):
@@ -421,6 +422,12 @@ class Context:
         out = np.zeros(8, dtype=np.uint64)
         self._check(self.lib.rtx_selftest_dmath(self.handle, _ptr(out), 8))
         return {"rsqrt": int(out[0]), "div3": int(out[1])}
+
+    def selftest_dmath_fast_paths(self):
+        """Mismatch counts of the unguarded fast paths (csrc/dmath.cuh): a wrong result without the range flag, or a wrong flag."""
+        out = np.zeros(8, dtype=np.uint64)
+        self._check(self.lib.rtx_selftest_dmath(self.handle, _ptr(out), 8))
+        return {k: int(out[i]) for i, k in enumerate(("sqrt", "rcp", "rsqrt", "div", "div_const"), start=2)}
 
     def debug_pixel(self, x, y):
         out = np.zeros(64, dtype=np.float32)

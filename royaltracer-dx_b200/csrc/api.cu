@@ -1070,6 +1070,7 @@ extern "C" rtx_status rtx_get_counters(rtx_ctx* c, rtx_counters* out) {
     TraceStats ts;
     RTX_CK(cudaMemcpy(&ts, c->d_stats, sizeof ts, cudaMemcpyDeviceToHost));
     out->nodes_visited = ts.nodes; out->tris_tested = ts.tris; out->instances_entered = ts.insts;
+    out->shading_replays = ts.replays;
     out->kernel_launches = c->launches;
     return RTX_OK;
 }

@@ -69,6 +69,7 @@ struct SceneAS {
 
 struct TraceStats {
     unsigned long long nodes, tris, insts;
+    unsigned long long replays;     // shading stages: paths replayed with IEEE operations (wavefront.cu)
 };
 
 }  // namespace rtx

@@ -128,132 +128,148 @@ __device__ __forceinline__ f3 SchlickFresnel(f3 F0, float cosTheta) {
     return saturate3(mk3(F0.x + (1.0f - F0.x) * p, F0.y + (1.0f - F0.y) * p, F0.z + (1.0f - F0.z) * p));
 }
 // :31-40
-__device__ __forceinline__ float D_GGX(float NdotH, float roughness) {
+template <class M = Ieee>
+__device__ __forceinline__ float D_GGX(float NdotH, float roughness, M m = M()) {
     float alpha = roughness * roughness;
     float alpha2 = alpha * alpha;
     float NdotH2 = NdotH * NdotH;
     float denom = (NdotH2 * (alpha2 - 1.0f) + 1.0f);
-    return alpha2 / ((RTX_PI_REF * denom) * denom);
+    return m.div(alpha2, (RTX_PI_REF * denom) * denom);
 }
 // :43-52
-__device__ __forceinline__ float G2_SmithGGX(float NdotV, float NdotL, float alpha) {
+template <class M = Ieee>
+__device__ __forceinline__ float G2_SmithGGX(float NdotV, float NdotL, float alpha, M m = M()) {
     float alpha2 = alpha * alpha;
-    float denomA = NdotV * sqrtf(alpha2 + ((1.0f - alpha2) * NdotL) * NdotL);
-    float denomB = NdotL * sqrtf(alpha2 + ((1.0f - alpha2) * NdotV) * NdotV);
-    return ((2.0f * NdotL) * NdotV) / (denomA + denomB);
+    float denomA = NdotV * m.sqrt(alpha2 + ((1.0f - alpha2) * NdotL) * NdotL);
+    float denomB = NdotL * m.sqrt(alpha2 + ((1.0f - alpha2) * NdotV) * NdotV);
+    return m.div((2.0f * NdotL) * NdotV, denomA + denomB);
 }
 // :55-61
-__device__ __forceinline__ float G1_SmithGGX(float NdotV, float alpha) {
+template <class M = Ieee>
+__device__ __forceinline__ float G1_SmithGGX(float NdotV, float alpha, M m = M()) {
     float alpha2 = alpha * alpha;
-    float denomC = sqrtf(alpha2 + ((1.0f - alpha2) * NdotV) * NdotV) + NdotV;
-    return (2.0f * NdotV) / denomC;
+    float denomC = m.sqrt(alpha2 + ((1.0f - alpha2) * NdotV) * NdotV) + NdotV;
+    return m.div(2.0f * NdotV, denomC);
 }
 // :65-76
-__device__ __forceinline__ void CoordinateSystem(f3 N, f3& T, f3& B) {
-    if (fabsf(N.z) < 0.999f) T = normalize3(cross3(mk3(0, 0, 1), N));
-    else T = normalize3(cross3(mk3(1, 0, 0), N));
+template <class M = Ieee>
+__device__ __forceinline__ void CoordinateSystem(f3 N, f3& T, f3& B, M m = M()) {
+    if (fabsf(N.z) < 0.999f) T = normalize3(cross3(mk3(0, 0, 1), N), m);
+    else T = normalize3(cross3(mk3(1, 0, 0), N), m);
     B = cross3(N, T);
 }
 // :93-169
-__device__ __forceinline__ f3 SampleBRDF_GGX(const MatOpt& mat, f3 outgoing, f3 normal, uint2& seed) {
+template <class M = Ieee>
+__device__ __forceinline__ f3 SampleBRDF_GGX(const MatOpt& mat, f3 outgoing, f3 normal, uint2& seed, M m = M()) {
     float alpha = hmul(mat.Pr, mat.Pr);
-    f3 N = normalize3(normal), V = normalize3(outgoing), T1, T2;
-    CoordinateSystem(N, T1, T2);
+    f3 N = normalize3(normal, m), V = normalize3(outgoing, m), T1, T2;
+    CoordinateSystem(N, T1, T2, m);
     float vx = dot3(T1, V), vy = dot3(T2, V), vz = dot3(N, V);
-    f3 Ve = normalize3(mk3(alpha * vx, alpha * vy, vz));
+    f3 Ve = normalize3(mk3(alpha * vx, alpha * vy, vz), m);
     float lensq = Ve.x * Ve.x + Ve.y * Ve.y;
-    f3 T1h = (lensq > 0.0f) ? mk3(-Ve.y, Ve.x, 0.0f) * d_rsqrt(lensq) : mk3(1, 0, 0);
+    f3 T1h = (lensq > 0.0f) ? mk3(-Ve.y, Ve.x, 0.0f) * m.rsqrt(lensq) : mk3(1, 0, 0);
     f3 T2h = cross3(Ve, T1h);
     float U1 = RandomFloat(seed), U2 = RandomFloat(seed);
-    float r = sqrtf(U1);
+    float r = m.sqrt(U1);
     float phi = (2.0f * RTX_PI_REF) * U2;
     float sn, cs; d_sincos(phi, &sn, &cs);
     float t1 = r * cs, t2 = r * sn;
     float s = 0.5f * (1.0f + Ve.z);
-    t2 = (1.0f - s) * sqrtf(saturate1(1.0f - t1 * t1)) + s * t2;
-    f3 Nh = (t1 * T1h + t2 * T2h) + sqrtf(saturate1((1.0f - t1 * t1) - t2 * t2)) * Ve;
-    f3 Ne = normalize3(mk3(alpha * Nh.x, alpha * Nh.y, fmaxf(0.0f, Nh.z)));
+    t2 = (1.0f - s) * m.sqrt(saturate1(1.0f - t1 * t1)) + s * t2;
+    f3 Nh = (t1 * T1h + t2 * T2h) + m.sqrt(saturate1((1.0f - t1 * t1) - t2 * t2)) * Ve;
+    f3 Ne = normalize3(mk3(alpha * Nh.x, alpha * Nh.y, fmaxf(0.0f, Nh.z)), m);
     f3 H = (Ne.x * T1 + Ne.y * T2) + Ne.z * N;
     f3 sample = reflect3(-V, H);
     if (dot3(sample, normal) < 0.0f) sample = -sample;
     return sample;
 }
 // :174-206
-__device__ __forceinline__ f3 EvaluateBRDF_GGX(const SceneData& S, const MatOpt& mat, f3 normal, f3 incoming, f3 outgoing) {
-    f3 N = normalize3(normal), V = normalize3(outgoing), L = normalize3(-incoming);
-    f3 H = normalize3(V + L);
+template <class M = Ieee>
+__device__ __forceinline__ f3 EvaluateBRDF_GGX(const SceneData& S, const MatOpt& mat, f3 normal, f3 incoming, f3 outgoing, M m = M()) {
+    f3 N = normalize3(normal, m), V = normalize3(outgoing, m), L = normalize3(-incoming, m);
+    f3 H = normalize3(V + L, m);
     float NdotV = dot3(N, V), NdotL = dot3(N, L), NdotH = dot3(N, H), VdotH = dot3(V, H);
     f3 F = SchlickFresnel(mat.Ks, VdotH);
-    float D = D_GGX(NdotH, mat.Pr);
-    float G = G2_SmithGGX(NdotV, NdotL, hmul(mat.Pr, mat.Pr));
+    float D = D_GGX(NdotH, mat.Pr, m);
+    float G = G2_SmithGGX(NdotV, NdotL, hmul(mat.Pr, mat.Pr), m);
     float denominator = (4.0f * NdotV) * NdotL;
     if (denominator < RTX_EPS) return mk3(0, 0, 0);
-    f3 specular = ((F * D) * G) / denominator;
+    f3 specular = m.div3((F * D) * G, denominator);
     float Ess = ESS_LUT(S, mat, NdotV);
-    float kms = (1.0f - Ess) / Ess;
+    float kms = m.div(1.0f - Ess, Ess);
     f3 specular_ess = specular * mk3(1.0f + mat.Ks.x * kms, 1.0f + mat.Ks.y * kms, 1.0f + mat.Ks.z * kms);
     if (any_nan_inf(specular_ess)) return mk3(0, 0, 0);
     return specular_ess;
 }
 // :209-224
-__device__ __forceinline__ float BRDF_PDF_GGX(const MatOpt& mat, f3 normal, f3 incoming, f3 outgoing) {
-    f3 N = normalize3(normal), V = normalize3(outgoing), L = normalize3(-incoming);
-    f3 H = normalize3(V + L);
+template <class M = Ieee>
+__device__ __forceinline__ float BRDF_PDF_GGX(const MatOpt& mat, f3 normal, f3 incoming, f3 outgoing, M m = M()) {
+    f3 N = normalize3(normal, m), V = normalize3(outgoing, m), L = normalize3(-incoming, m);
+    f3 H = normalize3(V + L, m);
     float NdotH = dot3(N, H), NdotV = dot3(N, V);
     float alpha = hmul(mat.Pr, mat.Pr);
-    float G1 = G1_SmithGGX(NdotV, alpha);
-    float D = D_GGX(NdotH, mat.Pr);
-    return (G1 * D) / (NdotV * 4.0f);
+    float G1 = G1_SmithGGX(NdotV, alpha, m);
+    float D = D_GGX(NdotH, mat.Pr, m);
+    return m.div(G1 * D, NdotV * 4.0f);
 }
 
 // ---- include/Lambertian_v6.hlsl
 // :2-37
-__device__ __forceinline__ f3 RandomUnitVectorInHemisphere(f3 normal, uint2& seed) {
+template <class M = Ieee>
+__device__ __forceinline__ f3 RandomUnitVectorInHemisphere(f3 normal, uint2& seed, M m = M()) {
     float u1 = RandomFloat(seed), u2 = RandomFloat(seed);
-    float r = sqrtf(u1);
+    float r = m.sqrt(u1);
     float theta = (2.0f * 3.14159265358979323846f) * u2;
     float sn, cs; d_sincos(theta, &sn, &cs);
     float x = r * cs, y = r * sn;
-    float z = sqrtf(fmaxf(0.0f, (1.0f - x * x) - y * y));
+    float z = m.sqrt(fmaxf(0.0f, (1.0f - x * x) - y * y));
     f3 h = normal;
     f3 up = fabsf(normal.z) < 0.999f ? mk3(0, 0, 1) : mk3(1, 0, 0);
-    f3 right = normalize3(cross3(up, h));
+    f3 right = normalize3(cross3(up, h), m);
     f3 forward = cross3(h, right);
     f3 hs = (x * right + y * forward) + z * h;
-    hs = normalize3(hs);
+    hs = normalize3(hs, m);
     if (dot3(hs, normal) < 0.0f) hs = -hs;
     return hs;
 }
 // :51-58, :61-64
-__device__ __forceinline__ f3 EvaluateBRDF_Lambertian(const MatOpt& mat) { return mat.Kd / RTX_PI_REF; }
-__device__ __forceinline__ float BRDF_PDF_Lambertian(f3 normal, f3 incoming) { return fmaxf(dot3(normal, -incoming), RTX_EPS) / RTX_PI_REF; }
+template <class M = Ieee>
+__device__ __forceinline__ f3 EvaluateBRDF_Lambertian(const MatOpt& mat, M m = M()) { return m.div3k(mat.Kd, RTX_PI_REF, RTX_RCP_PI_REF); }
+template <class M = Ieee>
+__device__ __forceinline__ float BRDF_PDF_Lambertian(f3 normal, f3 incoming, M m = M()) {
+    return m.divk(fmaxf(dot3(normal, -incoming), RTX_EPS), RTX_PI_REF, RTX_RCP_PI_REF);
+}
 
 // ---- shaders/BRDF_v7.hlsl
 // :50-70
-__device__ __forceinline__ void CalculateStrategyProbabilities(const SceneData& S, const MatOpt& mat, f3 outgoing, f3 normal, float& p_d, float& p_s) {
+template <class M = Ieee>
+__device__ __forceinline__ void CalculateStrategyProbabilities(const SceneData& S, const MatOpt& mat, f3 outgoing, f3 normal, float& p_d, float& p_s,
+                                                               M m = M()) {
     if (S.cfg_flags & RTX_FLAG_LAMBERT_ONLY) { p_d = 1.0f; p_s = 0.0f; return; }
     float cosTheta = dot3(normal, outgoing);
     f3 fr = SchlickFresnel(mat.Ks, cosTheta);
-    p_s = fminf(1.0f, ((fr.x + fr.y) + fr.z) / 3.0f + mat.Pm);
+    p_s = fminf(1.0f, m.divk((fr.x + fr.y) + fr.z, 3.0f, RTX_RCP_3) + mat.Pm);
     p_d = 1.0f - p_s;
 }
 // :7-48 (always one RandomFloat)
-__device__ __forceinline__ uint32_t SelectSamplingStrategy(const SceneData& S, const MatOpt& mat, f3 outgoing, f3 normal, uint2& seed) {
+template <class M = Ieee>
+__device__ __forceinline__ uint32_t SelectSamplingStrategy(const SceneData& S, const MatOpt& mat, f3 outgoing, f3 normal, uint2& seed, M m = M()) {
     float r = RandomFloat(seed);
     if (S.cfg_flags & RTX_FLAG_LAMBERT_ONLY) return 0;
     float cosTheta = dot3(normal, outgoing);
     f3 fr = SchlickFresnel(mat.Ks, cosTheta);
-    float p_s = fminf(1.0f, ((fr.x + fr.y) + fr.z) / 3.0f + mat.Pm);
+    float p_s = fminf(1.0f, m.divk((fr.x + fr.y) + fr.z, 3.0f, RTX_RCP_3) + mat.Pm);
     if (r <= p_s) { if (mat.Pr < 0.04f) return 0; return 1; }
     return 0;
 }
 // the two halves of SelectSamplingStrategy, for call sites that select twice at the same shading point
 // (Path_Sampler_v7.hlsl:118,196): p_s depends on (material, outgoing, normal) only.
-__device__ __forceinline__ float StrategyPs(const SceneData& S, const MatOpt& mat, f3 outgoing, f3 normal) {
+template <class M = Ieee>
+__device__ __forceinline__ float StrategyPs(const SceneData& S, const MatOpt& mat, f3 outgoing, f3 normal, M m = M()) {
     if (S.cfg_flags & RTX_FLAG_LAMBERT_ONLY) return -1.0f;          // r <= p_s never holds: always strategy 0
     float cosTheta = dot3(normal, outgoing);
     f3 fr = SchlickFresnel(mat.Ks, cosTheta);
-    return fminf(1.0f, ((fr.x + fr.y) + fr.z) / 3.0f + mat.Pm);
+    return fminf(1.0f, m.divk((fr.x + fr.y) + fr.z, 3.0f, RTX_RCP_3) + mat.Pm);
 }
 __device__ __forceinline__ uint32_t SelectWithPs(float p_s, const MatOpt& mat, uint2& seed) {
     float r = RandomFloat(seed);
@@ -261,9 +277,10 @@ __device__ __forceinline__ uint32_t SelectWithPs(float p_s, const MatOpt& mat, u
     return 0;
 }
 // :74-88
-__device__ __forceinline__ f3 SampleBRDF(uint32_t strategy, const MatOpt& mat, f3 outgoing, f3 normal, uint2& seed) {
-    if (strategy == 0) return RandomUnitVectorInHemisphere(normal, seed);
-    return SampleBRDF_GGX(mat, outgoing, normal, seed);
+template <class M = Ieee>
+__device__ __forceinline__ f3 SampleBRDF(uint32_t strategy, const MatOpt& mat, f3 outgoing, f3 normal, uint2& seed, M m = M()) {
+    if (strategy == 0) return RandomUnitVectorInHemisphere(normal, seed, m);
+    return SampleBRDF_GGX(mat, outgoing, normal, seed, m);
 }
 // :109-124
 __device__ __forceinline__ float BRDF_PDF(uint32_t strategy, const MatOpt& mat, f3 normal, f3 incidence, f3 outgoing) {
@@ -271,9 +288,10 @@ __device__ __forceinline__ float BRDF_PDF(uint32_t strategy, const MatOpt& mat, 
     return BRDF_PDF_GGX(mat, normal, incidence, outgoing);
 }
 // the combined lobe F = p_d*f0 + p_s*f1 (Sampler_v7.hlsl:123-128,248-261,361-374,443-456,601-614; Path_Sampler_v7.hlsl:66-78)
-__device__ __forceinline__ f3 CombinedF(const SceneData& S, const MatOpt& mat, f3 normal, f3 incidence, f3 outgoing, float p_d, float p_s) {
-    f3 F1 = SafeMultiply(p_d, EvaluateBRDF_Lambertian(mat));
-    f3 F2 = (S.cfg_flags & RTX_FLAG_LAMBERT_ONLY) ? mk3(0, 0, 0) : SafeMultiply(p_s, EvaluateBRDF_GGX(S, mat, normal, incidence, outgoing));
+template <class M = Ieee>
+__device__ __forceinline__ f3 CombinedF(const SceneData& S, const MatOpt& mat, f3 normal, f3 incidence, f3 outgoing, float p_d, float p_s, M m = M()) {
+    f3 F1 = SafeMultiply(p_d, EvaluateBRDF_Lambertian(mat, m));
+    f3 F2 = (S.cfg_flags & RTX_FLAG_LAMBERT_ONLY) ? mk3(0, 0, 0) : SafeMultiply(p_s, EvaluateBRDF_GGX(S, mat, normal, incidence, outgoing, m));
     return F1 + F2;
 }
 // combined pdf with a common scale applied to each lobe before SafeMultiply: P = SM(p_d, pdf0*a/b) + SM(p_s, pdf1*a/b)
@@ -309,11 +327,12 @@ struct LobeCtx {
 };
 // N = normalize3(normal) and V = normalize3(outgoing) supplied by the caller (call sites that build two contexts at one
 // vertex share N, and often already hold V)
-__device__ __forceinline__ LobeCtx make_lobe_ctx_nv(const SceneData& S, const MatOpt& mat, f3 normal, f3 N, f3 V, float p_d, float p_s) {
+template <class M = Ieee>
+__device__ __forceinline__ LobeCtx make_lobe_ctx_nv(const SceneData& S, const MatOpt& mat, f3 normal, f3 N, f3 V, float p_d, float p_s, M m = M()) {
     LobeCtx c;
     c.normal = normal; c.p_d = p_d; c.p_s = p_s;
     c.lambert_only = (S.cfg_flags & RTX_FLAG_LAMBERT_ONLY) != 0u;
-    c.F1 = SafeMultiply(p_d, EvaluateBRDF_Lambertian(mat));
+    c.F1 = SafeMultiply(p_d, EvaluateBRDF_Lambertian(mat, m));
     c.Ks = mat.Ks;
     if (!c.lambert_only) {
         c.N = N; c.V = V;
@@ -323,58 +342,61 @@ __device__ __forceinline__ LobeCtx make_lobe_ctx_nv(const SceneData& S, const Ma
         c.a2D = alphaD * alphaD; c.a2Dm1 = c.a2D - 1.0f;
         const float alphaG = hmul(mat.Pr, mat.Pr);
         c.a2G = alphaG * alphaG; c.oma2G = 1.0f - c.a2G;
-        c.sV = sqrtf(c.a2G + (c.oma2G * c.NdotV) * c.NdotV);
-        c.G1 = (2.0f * c.NdotV) / (c.sV + c.NdotV);
+        c.sV = m.sqrt(c.a2G + (c.oma2G * c.NdotV) * c.NdotV);
+        c.G1 = m.div(2.0f * c.NdotV, c.sV + c.NdotV);
         const float Ess = ESS_LUT(S, mat, c.NdotV);
-        const float kms = (1.0f - Ess) / Ess;
+        const float kms = m.div(1.0f - Ess, Ess);
         c.essScale = mk3(1.0f + mat.Ks.x * kms, 1.0f + mat.Ks.y * kms, 1.0f + mat.Ks.z * kms);
     }
     return c;
 }
-__device__ __forceinline__ LobeCtx make_lobe_ctx(const SceneData& S, const MatOpt& mat, f3 normal, f3 outgoing, float p_d, float p_s) {
+template <class M = Ieee>
+__device__ __forceinline__ LobeCtx make_lobe_ctx(const SceneData& S, const MatOpt& mat, f3 normal, f3 outgoing, float p_d, float p_s, M m = M()) {
     const bool lo = (S.cfg_flags & RTX_FLAG_LAMBERT_ONLY) != 0u;
-    return make_lobe_ctx_nv(S, mat, normal, lo ? normal : normalize3(normal), lo ? outgoing : normalize3(outgoing), p_d, p_s);
+    return make_lobe_ctx_nv(S, mat, normal, lo ? normal : normalize3(normal, m), lo ? outgoing : normalize3(outgoing, m), p_d, p_s, m);
 }
 // F = CombinedF(...), P = CombinedP(...) (scaled == false) or CombinedP_scaled(..., a, b) for one incidence direction.
-template <bool WANT_F, bool WANT_P>
-__device__ __forceinline__ void lobe_FP(const LobeCtx& c, f3 incidence, bool scaled, float a, float b, f3& F, float& P) {
+template <bool WANT_F, bool WANT_P, class M = Ieee>
+__device__ __forceinline__ void lobe_FP(const LobeCtx& c, f3 incidence, bool scaled, float a, float b, f3& F, float& P, M m = M()) {
     f3 F2 = mk3(0, 0, 0); float P2 = 0.0f;
     if (!c.lambert_only) {
-        const f3 L = normalize3(-incidence);
-        const f3 H = normalize3(c.V + L);
+        const f3 L = normalize3(-incidence, m);
+        const f3 H = normalize3(c.V + L, m);
         const float NdotH = dot3(c.N, H);
         const float denomD = (NdotH * NdotH) * c.a2Dm1 + 1.0f;
-        const float D = c.a2D / ((RTX_PI_REF * denomD) * denomD);                // D_GGX
+        const float D = m.div(c.a2D, (RTX_PI_REF * denomD) * denomD);           // D_GGX
         if (WANT_F) {
             const float NdotL = dot3(c.N, L), VdotH = dot3(c.V, H);
             const f3 Fr = SchlickFresnel(c.Ks, VdotH);
-            const float denomA = c.NdotV * sqrtf(c.a2G + (c.oma2G * NdotL) * NdotL);
+            const float denomA = c.NdotV * m.sqrt(c.a2G + (c.oma2G * NdotL) * NdotL);
             const float denomB = NdotL * c.sV;
-            const float G = ((2.0f * NdotL) * c.NdotV) / (denomA + denomB);      // G2_SmithGGX
+            const float G = m.div((2.0f * NdotL) * c.NdotV, denomA + denomB);   // G2_SmithGGX
             const float denominator = c.NdotV4 * NdotL;
             f3 spec = mk3(0, 0, 0);
             if (!(denominator < RTX_EPS)) {
-                spec = (((Fr * D) * G) / denominator) * c.essScale;
+                spec = m.div3((Fr * D) * G, denominator) * c.essScale;
                 if (any_nan_inf(spec)) spec = mk3(0, 0, 0);
             }
             F2 = SafeMultiply(c.p_s, spec);
         }
         if (WANT_P) {
-            float pdf = (c.G1 * D) / c.NdotV4;                                    // BRDF_PDF_GGX (NdotV*4 == 4*NdotV)
-            if (scaled) pdf = (pdf * a) / b;
+            float pdf = m.div(c.G1 * D, c.NdotV4);                                // BRDF_PDF_GGX (NdotV*4 == 4*NdotV)
+            if (scaled) pdf = m.div(pdf * a, b);
             P2 = SafeMultiply1(c.p_s, pdf);
         }
     }
     if (WANT_F) F = c.F1 + F2;
     if (WANT_P) {
-        float pl = BRDF_PDF_Lambertian(c.normal, incidence);
-        if (scaled) pl = (pl * a) / b;
+        float pl = BRDF_PDF_Lambertian(c.normal, incidence, m);
+        if (scaled) pl = m.div(pl * a, b);
         P = SafeMultiply1(c.p_d, pl) + P2;
     }
 }
 
 // ---- ClosestHit, shaders/Hit_v7.hlsl:12-61 (area is not carried: nothing on the E0 path reads payload.area)
-__device__ __forceinline__ void ClosestHit(const SceneData& S, f3 ro, f3 rd, float t, float b1, float b2, uint32_t prim, uint32_t inst, HitInfo& p) {
+template <class MP = Ieee>
+__device__ __forceinline__ void ClosestHit(const SceneData& S, f3 ro, f3 rd, float t, float b1, float b2, uint32_t prim, uint32_t inst, HitInfo& p,
+                                           MP m = MP()) {
     const ModelRef M = S.models[S.inst_model[inst]];
     p.objID = inst;
     f3 worldOrigin = ro + t * rd;
@@ -392,7 +414,7 @@ __device__ __forceinline__ void ClosestHit(const SceneData& S, f3 ro, f3 rd, flo
     }
     f3 e1 = pos[1] - pos[0], e2 = pos[2] - pos[0];
     f3 cross_a = cross3(e1, e2);
-    f3 flatNormal = normalize3(cross_a);
+    f3 flatNormal = normalize3(cross_a, m);
     f3 smooth = mk3(0, 0, 0);
 #pragma unroll
     for (int i = 0; i < 3; i++) {
@@ -400,33 +422,35 @@ __device__ __forceinline__ void ClosestHit(const SceneData& S, f3 ro, f3 rd, flo
         else smooth = smooth + flatNormal * bary[i];
     }
     f3 normal;
-    if (length3(smooth) > 0.0001f) normal = normalize3(smooth); else normal = flatNormal;
+    if (length3(smooth, m) > 0.0001f) normal = normalize3(smooth, m); else normal = flatNormal;
     f3 wn = mul43(S.props[inst].objectToWorldNormal, normal.x, normal.y, normal.z, 0.0f);
-    p.hitNormal = normalize3(wn);
+    p.hitNormal = normalize3(wn, m);
     p.materialID = materialID;
     p.hitPosition = worldOrigin;
 }
 
 // ---- shaders/Sampler_v7.hlsl
 // :106-131
-__device__ __forceinline__ f3 ReconnectDI(const SceneData& S, f3 x1, f3 n1, f3 x2, f3 n2, f3 L, f3 outgoing, const MatOpt& material) {
+template <class M = Ieee>
+__device__ __forceinline__ f3 ReconnectDI(const SceneData& S, f3 x1, f3 n1, f3 x2, f3 n2, f3 L, f3 outgoing, const MatOpt& material, M m = M()) {
     f3 dir = x2 - x1;
-    float dist = length3(dir);
-    float cosThetaX1 = fmaxf(0.0f, dot3(n1, normalize3(dir)));
-    if (dot3(n2, normalize3(-dir)) < 0.0f) n2 = -n2;
-    float cosThetaX2 = fmaxf(0.0f, dot3(n2, normalize3(-dir)));
+    float dist = length3(dir, m);
+    float cosThetaX1 = fmaxf(0.0f, dot3(n1, normalize3(dir, m)));
+    if (dot3(n2, normalize3(-dir, m)) < 0.0f) n2 = -n2;
+    float cosThetaX2 = fmaxf(0.0f, dot3(n2, normalize3(-dir, m)));
     float p_d, p_s;
-    CalculateStrategyProbabilities(S, material, normalize3(outgoing), n1, p_d, p_s);
-    f3 F = CombinedF(S, material, n1, normalize3(-dir), normalize3(outgoing), p_d, p_s);
-    return (((F * L) * cosThetaX1) * cosThetaX2) / (dist * dist);
+    CalculateStrategyProbabilities(S, material, normalize3(outgoing, m), n1, p_d, p_s, m);
+    f3 F = CombinedF(S, material, n1, normalize3(-dir, m), normalize3(outgoing, m), p_d, p_s, m);
+    return m.div3(((F * L) * cosThetaX1) * cosThetaX2, dist * dist);
 }
 // :134-161
-__device__ __forceinline__ f3 ReconnectGI(const SceneData& S, f3 x1, f3 n1, f3 x2, f3 L, f3 outgoing, const MatOpt& material1) {
+template <class M = Ieee>
+__device__ __forceinline__ f3 ReconnectGI(const SceneData& S, f3 x1, f3 n1, f3 x2, f3 L, f3 outgoing, const MatOpt& material1, M m = M()) {
     f3 dir = x2 - x1;
-    float cosThetaX1 = fabsf(dot3(n1, normalize3(dir)));
+    float cosThetaX1 = fabsf(dot3(n1, normalize3(dir, m)));
     float p_d, p_s;
-    CalculateStrategyProbabilities(S, material1, normalize3(outgoing), n1, p_d, p_s);
-    f3 Fx1 = CombinedF(S, material1, n1, normalize3(-dir), normalize3(outgoing), p_d, p_s);
+    CalculateStrategyProbabilities(S, material1, normalize3(outgoing, m), n1, p_d, p_s, m);
+    f3 Fx1 = CombinedF(S, material1, n1, normalize3(-dir, m), normalize3(outgoing, m), p_d, p_s, m);
     f3 fr = (Fx1 * cosThetaX1) * L;
     if (any_nan_inf(fr)) return mk3(0, 0, 0);
     return fr;
@@ -446,7 +470,8 @@ __device__ __forceinline__ uint32_t SelectLight(const SceneData& S, float random
 struct LightSample { f3 point, normal_l, L_norm, emission; float dist2, pdf_l; };
 
 // shared front half of SampleLightNEE (:292-346) and SampleLightNEE_GI (:529-584): 3 RandomFloat
-__device__ __forceinline__ void SampleLightPoint(const SceneData& S, f3 origin, uint2& seed, LightSample& ls) {
+template <class MP = Ieee>
+__device__ __forceinline__ void SampleLightPoint(const SceneData& S, f3 origin, uint2& seed, LightSample& ls, MP m = MP()) {
     float randomValue = RandomFloat(seed);
     const float4* lt = reinterpret_cast<const float4*>(S.lights + SelectLight(S, randomValue));
     const float4 l0 = __ldg(lt), l1 = __ldg(lt + 1), l2 = __ldg(lt + 2), l3 = __ldg(lt + 3);
@@ -460,13 +485,13 @@ __device__ __forceinline__ void SampleLightPoint(const SceneData& S, f3 origin, 
     ls.point = (u * x_v + v * y_v) + w * z_v;
     f3 L = ls.point - origin;
     ls.dist2 = dot3(L, L);
-    ls.L_norm = normalize3(L);
+    ls.L_norm = normalize3(L, m);
     f3 cross_l = cross3(y_v - x_v, z_v - x_v);
-    f3 normal_l = normalize3(cross_l);
+    f3 normal_l = normalize3(cross_l, m);
     if (dot3(normal_l, -ls.L_norm) < 0.0f) normal_l = -normal_l;
     ls.normal_l = normal_l;
-    float area_l = fabsf(length3(cross_l) * 0.5f);
-    ls.pdf_l = l2.w / fmaxf(area_l, RTX_EPS);
+    float area_l = fabsf(length3(cross_l, m) * 0.5f);
+    ls.pdf_l = m.div(l2.w, fmaxf(area_l, RTX_EPS));
     ls.emission = mk3(l3.x, l3.y, l3.z);
 }
 
