@@ -49,7 +49,6 @@ typedef struct { float t, u, v; uint32_t prim; uint32_t inst; } rtx_hit;      /*
 
 #define RTX_FLAG_JITTER          1u  /* 2 RandomFloat draws before anything else (legacy include/RayGen.hlsl:84-85) */
 #define RTX_FLAG_LAMBERT_ONLY    2u  /* strategy probabilities forced to (1,0) (BASELINE config C1) */
-#define RTX_FLAG_SORT_MATERIAL   4u  /* bin shading queues by material id */
 #define RTX_FLAG_LEGACY_RR       16u /* rtx_render_pass runs the reference's legacy estimator (include/RayGen.hlsl:60-137 + include/Hit.hlsl:
                                        * RIS-10 NEE with one shadow ray per bounce, MIS on emitter hits, Russian roulette after depth 3);
                                        * cfg.bounces (<= 60) caps the number of closest-hit rays per path */
@@ -68,7 +67,7 @@ typedef struct {
     uint32_t bounces;           /* Common_v7.hlsl:11, default 3 */
     uint32_t nee_samples;       /* Common_v7.hlsl:8,  default 4 */
     uint32_t nee_samples_di;    /* Common_v7.hlsl:9,  default 4 */
-    uint32_t flags;
+    uint32_t flags;             /* RTX_FLAG_*; rtx_create rejects any other bit */
     uint32_t samples_per_pass;  /* paths in flight per DispatchRays-equivalent = W*H*samples_per_pass (>=1) */
     void*    stream;            /* cudaStream_t to run on, NULL = context-owned stream */
 } rtx_config;
@@ -168,8 +167,7 @@ rtx_status rtx_last_pass_ms(rtx_ctx*, float* trace_ms, float* total_ms);
 #define RTX_STAGE_SCATTER 6
 #define RTX_STAGE_FINALIZE 7
 #define RTX_STAGE_ACCUMULATE 8
-#define RTX_STAGE_SORT 9
-#define RTX_STAGE_COUNT 10
+#define RTX_STAGE_COUNT 9
 rtx_status rtx_last_pass_stage_ms(rtx_ctx*, float* ms_by_stage, uint32_t n_stages, float* total_ms);
 /* runtime options.  RTX_OPT_TRACE_STATS: closest-hit traversals of rtx_render_pass also count nodes/triangles/instances
  * (instrumented kernel variant: for the roofline's B_ray, never for timed runs), and the shading stages count the paths they

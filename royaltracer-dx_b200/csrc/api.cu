@@ -139,6 +139,8 @@ extern "C" rtx_status rtx_create(const rtx_config* cfg, rtx_ctx** out) {
     if (!cfg || !out) return fail(RTX_ERR_ARG, "rtx_create: null argument");
     if (cfg->struct_size != sizeof(rtx_config)) return fail(RTX_ERR_ARG, "rtx_create: rtx_config.struct_size mismatch");
     if (cfg->width == 0 || cfg->height == 0) return fail(RTX_ERR_ARG, "rtx_create: zero-sized image");
+    if (cfg->flags & ~(RTX_FLAG_JITTER | RTX_FLAG_LAMBERT_ONLY | RTX_FLAG_RESTIR | RTX_FLAG_LEGACY_RR | RTX_FLAG_FAST_MATH))
+        return fail(RTX_ERR_ARG, "rtx_create: unknown flags (valid: RTX_FLAG_JITTER | RTX_FLAG_LAMBERT_ONLY | RTX_FLAG_RESTIR | RTX_FLAG_LEGACY_RR | RTX_FLAG_FAST_MATH)");
     // every path range owns a block of 128 queue counters of which the indirect queues take 5 + bounces (wavefront.cu); the legacy
     // estimator keeps its per-bounce bookkeeping in 64 slots (legacy.cu)
     if ((cfg->flags & RTX_FLAG_LEGACY_RR) ? cfg->bounces > 60u : cfg->bounces > 120u)
@@ -379,7 +381,7 @@ static rtx_status sync_frame_state(rtx_ctx* c) {
 // is the call part of a per-frame loop that can be pipelined?  (the previous frame ended with rtx_render_pass [+ read-back] and nothing else)
 static bool frame_fast_ok(rtx_ctx* c) {
     return c->pipeline && c->frame_pipeline && c->frame_seq_ok && c->wb_ready &&
-           !(c->cfg.flags & (RTX_FLAG_LEGACY_RR | RTX_FLAG_RESTIR | RTX_FLAG_SORT_MATERIAL)) && !c->timing.stage_timing && !c->trace_stats &&
+           !(c->cfg.flags & (RTX_FLAG_LEGACY_RR | RTX_FLAG_RESTIR)) && !c->timing.stage_timing && !c->trace_stats &&
            (uint64_t)c->cfg.width * c->cfg.height * c->cfg.samples_per_pass >= 65536u && lane_buffers(c) && ensure_frame_set(c);
 }
 
@@ -619,7 +621,7 @@ extern "C" rtx_status rtx_render_pass(rtx_ctx* c, uint32_t first_sample, uint32_
     SceneAS AS = make_as(c);
     const uint32_t npx = c->cfg.width * c->cfg.height;
     // pipelined passes (see rtx_ctx): the estimator E0 without per-launch instrumentation, frames large enough to be cut into path ranges
-    const bool eligible = c->pipeline && !(c->cfg.flags & (RTX_FLAG_LEGACY_RR | RTX_FLAG_RESTIR | RTX_FLAG_SORT_MATERIAL)) &&
+    const bool eligible = c->pipeline && !(c->cfg.flags & (RTX_FLAG_LEGACY_RR | RTX_FLAG_RESTIR)) &&
                           !c->timing.stage_timing && !c->trace_stats && (uint64_t)npx * c->cfg.samples_per_pass >= 65536u && lane_buffers(c);
     uint32_t done = 0;
     while (done < n_samples) {

@@ -67,7 +67,10 @@ __device__ __forceinline__ MatOpt load_matopt(const SceneData& S, uint32_t id, f
 }
 
 // shaders/Common_v7.hlsl:119-138
-__device__ __forceinline__ uint2 tea4_body(uint2 seed) {
+// One out-of-line copy per kernel: the shading stages draw ~20 numbers per bounce, inlined that is ~1200 of k_gi_step's 4000 SASS
+// instructions, and the kernel stalls on instruction fetch (ncu: no_instruction 1.65 stall cycles per issue).  k_gi_step 3.78 -> 3.70 ms
+// per C2 pass (profiles/r02_s1_stage_times.txt).
+static __device__ __noinline__ uint2 tea4(uint2 seed) {
     uint32_t v0 = seed.x, v1 = seed.y, sum = 0u;
 #pragma unroll
     for (int i = 0; i < 4; i++) {
@@ -77,14 +80,6 @@ __device__ __forceinline__ uint2 tea4_body(uint2 seed) {
     }
     return make_uint2(v0, v1);
 }
-// One out-of-line copy per kernel: the shading stages draw ~20 numbers per bounce, inlined that is ~1200 of k_gi_step's 4000 SASS
-// instructions, and the kernel stalls on instruction fetch (ncu: no_instruction 1.65 stall cycles per issue).  k_gi_step 3.78 -> 3.70 ms
-// per C2 pass (profiles/r02_s1_stage_times.txt); -DRTX_TEA_INLINE restores the inlined form.
-#ifdef RTX_TEA_INLINE
-__device__ __forceinline__ uint2 tea4(uint2 seed) { return tea4_body(seed); }
-#else
-static __device__ __noinline__ uint2 tea4(uint2 seed) { return tea4_body(seed); }
-#endif
 __device__ __forceinline__ float RandomFloat(uint2& seed) {
     seed = tea4(seed);
     return (float)seed.x / 4294967296.0f;
@@ -281,11 +276,6 @@ template <class M = Ieee>
 __device__ __forceinline__ f3 SampleBRDF(uint32_t strategy, const MatOpt& mat, f3 outgoing, f3 normal, uint2& seed, M m = M()) {
     if (strategy == 0) return RandomUnitVectorInHemisphere(normal, seed, m);
     return SampleBRDF_GGX(mat, outgoing, normal, seed, m);
-}
-// :109-124
-__device__ __forceinline__ float BRDF_PDF(uint32_t strategy, const MatOpt& mat, f3 normal, f3 incidence, f3 outgoing) {
-    if (strategy == 0) return BRDF_PDF_Lambertian(normal, incidence);
-    return BRDF_PDF_GGX(mat, normal, incidence, outgoing);
 }
 // the combined lobe F = p_d*f0 + p_s*f1 (Sampler_v7.hlsl:123-128,248-261,361-374,443-456,601-614; Path_Sampler_v7.hlsl:66-78)
 template <class M = Ieee>

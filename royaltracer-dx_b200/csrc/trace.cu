@@ -27,18 +27,8 @@ namespace rtx {
 #define RTX_SCHED_DEFAULT 0x060808   // th_tri | th_inst << 8 | th_node << 16: run the triangle (instance) phase when >= th lanes are parked,
 #endif                               // or whenever fewer than th_node lanes have node work left (sweep: profiles/r01_s4_sched_sweep.txt)
 
-// rays are read once and hit records are read a launch later: evict-first loads / stores, so that the launch's own streaming traffic does
-// not push the BVH out of the L2 (wave_dev.cuh StateView::ld has the numbers; -DRTX_STREAM_HINTS=0 restores plain accesses)
-#ifndef RTX_STREAM_HINTS
-#define RTX_STREAM_HINTS 1
-#endif
-#if RTX_STREAM_HINTS
-#define RTX_ST(P, V) __stcs((P), (V))
-#define RTX_LD_RAY(P) __ldcs(P)
-#else
-#define RTX_ST(P, V) (*(P) = (V))
-#define RTX_LD_RAY(P) __ldg(P)
-#endif
+// rays are read once and hit records are read a launch later: evict-first loads / stores (__ldcs / __stcs), so that the launch's own
+// streaming traffic does not push the BVH out of the L2 (wave_dev.cuh StateView::ld has the numbers)
 
 template <bool ANY_HIT, bool STATS>
 __global__ void __launch_bounds__(TRACE_BLOCK, RTX_TRACE_MINB)
@@ -90,7 +80,7 @@ trace_kernel(SceneAS S, const float4* __restrict__ o_tmin, const float4* __restr
             const uint32_t mine = base + (uint32_t)__popc(idle & lt_mask);
             if (!active && mine < n) {
                 const uint32_t slot = order ? __ldg(order + (mine < n_heavy ? mine : cap - 1u - (mine - n_heavy))) : mine;
-                trav_init(T, C, S, RTX_LD_RAY(o_tmin + slot), RTX_LD_RAY(d_tmax + slot), slot);
+                trav_init(T, C, S, __ldcs(o_tmin + slot), __ldcs(d_tmax + slot), slot);
                 active = true;
             }
         }
@@ -126,14 +116,14 @@ trace_kernel(SceneAS S, const float4* __restrict__ o_tmin, const float4* __restr
 #define RTX_WRITE_RESULT                                                                                       \
             {                                                                                                  \
                 const uint32_t j = __float_as_uint(C.wo->w);                                                   \
-                if (!ANY_HIT) { const float4 h = *C.hit; RTX_ST(hit_a + j, make_float4(T.ht, h.x, h.y, h.z)); } \
+                if (!ANY_HIT) { const float4 h = *C.hit; __stcs(hit_a + j, make_float4(T.ht, h.x, h.y, h.z)); } \
                 /* any-hit with a visibility array: an occluded ray clears its path's entry (no scatter kernel) */ \
                 if (ANY_HIT && vis) { if (T.hinst != 0xFFFFFFFFu) vis[__ldg(vis_pid + j)] = 0.0f; }            \
                 /* ... or sets bit (pid & 15) of word pid >> 4 of an occlusion mask (the ReSTIR reuse passes) */   \
                 else if (ANY_HIT && vmask) {                                                                   \
                     if (T.hinst != 0xFFFFFFFFu) { const uint32_t pid = __ldg(vis_pid + j); atomicOr(&vmask[pid >> 4], 1u << (pid & 15u)); } \
                 }                                                                                              \
-                else RTX_ST(hit_inst + j, T.hinst);                                                            \
+                else __stcs(hit_inst + j, T.hinst);                                                            \
             }
             if (pend == PEND_TRI) {
                 if (do_tri) {

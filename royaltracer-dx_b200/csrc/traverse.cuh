@@ -32,33 +32,12 @@ namespace rtx {
         else *S.overflow = 1u;                                        \
     } while (0)
 
-#ifndef RTX_CONV_MODE
-#define RTX_CONV_MODE 1     // 0: shift+or (1 + q/256), 1: byte permute (1 + q*2^-15), 2: fp16 pairs (1024 + q)
-#endif
-
-__device__ __forceinline__ uint32_t sign_extend_s8x4(uint32_t x) {
-    uint32_t d;
-    asm("prmt.b32 %0, %1, %2, %3;" : "=r"(d) : "r"(x), "r"(0u), "r"(0xba98u));
-    return d;
-}
-__device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel) {
-    uint32_t d;
-    asm("prmt.b32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(sel));
-    return d;
-}
-__device__ __forceinline__ void prefetch_l1(const void* p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
-__device__ __forceinline__ uint32_t extract_byte(uint32_t x, int i) { return (x >> (i * 8)) & 0xffu; }
-
-// byte i of x as a float that is affine in q (see RTX_CONV_MODE); the matching (scale, offset) are in plane_coeffs()
+// byte I of x as the float 1 + q*2^-15 (0x3F80qq00: one byte permute with `one` = 0x3F800000); intersect_node() scales it back
 template <int I>
 __device__ __forceinline__ float plane_byte(uint32_t x, uint32_t one) {
-#if RTX_CONV_MODE == 0
-    return __uint_as_float(0x3F800000u | (((x >> (I * 8)) & 0xffu) << 15));     // 1 + q/256
-#else
-    uint32_t d;                                                                  // 0x3F80qq00 = 1 + q*2^-15
+    uint32_t d;
     asm("prmt.b32 %0, %1, %2, %3;" : "=r"(d) : "r"(x), "r"(one), "n"(0x7604 | (I << 4)));
     return __uint_as_float(d);
-#endif
 }
 
 struct RaySpace {          // the ray in the space currently traversed + derived constants
@@ -68,8 +47,6 @@ struct RaySpace {          // the ray in the space currently traversed + derived
     uint32_t ksel;         // one-hot axis selectors: bit (3a + c) set iff k_a == c, a = 0 (kx), 1 (ky), 2 (kz)
     uint32_t octinv4;      // (dx>=0 | dy>=0 <<1 | dz>=0 <<2) * 0x01010101
 };
-
-__device__ __forceinline__ float sel3(float x, float y, float z, uint32_t k) { return k == 0 ? x : (k == 1 ? y : z); }
 
 __device__ __forceinline__ float rcp_approx(float x) {
     float r;
@@ -187,23 +164,14 @@ __device__ __forceinline__ uint32_t intersect_node(const RaySpace& r, uint4 n0, 
     const float ax = __uint_as_float((e & 0xffu) << 23) * r.ix;
     const float ay = __uint_as_float(((e >> 8) & 0xffu) << 23) * r.iy;
     const float az = __uint_as_float(((e >> 16) & 0xffu) << 23) * r.iz;
-    // plane = p + q * 2^e  ->  t = F(q) * A + B with F(q) = 1 + q/S the float plane_byte() builds, A = S a, B = b - A.
-#if RTX_CONV_MODE == 0
-    const float SC = 256.0f;
-#else
+    // plane = p + q * 2^e  ->  t = F(q) * A + B with F(q) = 1 + q/2^15 the float plane_byte() builds, A = 2^15 a, B = b - A.
     const float SC = 32768.0f;
-#endif
     const float ax2 = ax * SC, ay2 = ay * SC, az2 = az * SC;
     const float bx = (px - r.ox) * r.ix - ax2, by = (py - r.oy) * r.iy - ay2, bz = (pz - r.oz) * r.iz - az2;
-#if RTX_CONV_MODE == 0
-    // the rounding of (b - 256 a) is 2^-16 of a grid cell: inside the builder's padding
-    const float bxn = bx, bxf = bx, byn = by, byf = by, bzn = bz, bzf = bz;
-#else
     // the rounding of (b - 2^15 a) is up to 2^-9 of a grid cell: widen the slab interval by 2^-23 |A| (= 2^-8 cell) instead
     const float w = 1.1920929e-7f, fx = fabsf(ax2), fy = fabsf(ay2), fz = fabsf(az2);
     const float bxn = __fmaf_rn(fx, -w, bx), bxf = __fmaf_rn(fx, w, bx), byn = __fmaf_rn(fy, -w, by), byf = __fmaf_rn(fy, w, by);
     const float bzn = __fmaf_rn(fz, -w, bz), bzf = __fmaf_rn(fz, w, bz);
-#endif
     const bool nx = !(r.octinv4 & 1u), ny = !(r.octinv4 & 2u), nz = !(r.octinv4 & 4u);
     const uint32_t WI = n1.z;
     uint32_t acc = 0;

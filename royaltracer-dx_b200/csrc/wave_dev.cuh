@@ -8,28 +8,18 @@ struct StateView {
     float4* base; uint32_t n;
     uint2* seed;          // the path's RNG state in its own 8-byte plane: every stage updates it, and as the .w of two float4 planes it cost a
                           // 32-byte read and a 32-byte write per path and stage to move 8 bytes (E0 stages only; nullptr elsewhere)
-#ifdef RTX_STATE_AOS
-    // one 288-byte record per path (9 whole 32-byte sectors): a thread's accesses use every byte of the sectors it touches whatever the
-    // order of the path ids in its warp — queues that are not in pixel order (two-ended LPT queues, material bins) cost no extra sectors
-    __device__ __forceinline__ float4& at(int plane, uint32_t pid) const { return base[(size_t)pid * NSTATE + plane]; }
-#else
     __device__ __forceinline__ float4& at(int plane, uint32_t pid) const { return base[(size_t)plane * n + pid]; }
-#endif
     // The path state is STREAMED: each stage reads a plane once and the next reader is a launch later, ~0.5 GB per k_gi_step launch.
     // ld / stt use the evict-first cache policy (ld.global.cs / st.global.cs) so that this traffic does not push the BVH, which every
     // traversal launch re-reads at random, out of the L2: closest-hit launches -2.7 %, C2 pass -1.3 % (profiles/r02_l2_policy_ab.txt).
-    // -DRTX_STREAM_HINTS=0 restores plain accesses.
-#ifndef RTX_STREAM_HINTS
-#define RTX_STREAM_HINTS 1
-#endif
-    __device__ __forceinline__ float4 ld(int plane, uint32_t pid) const { return RTX_STREAM_HINTS ? __ldcs(&at(plane, pid)) : at(plane, pid); }
-    __device__ __forceinline__ void stt(int plane, uint32_t pid, float4 v) const { if (RTX_STREAM_HINTS) __stcs(&at(plane, pid), v); else at(plane, pid) = v; }
-    __device__ __forceinline__ uint2 ld_seed(uint32_t pid) const { return RTX_STREAM_HINTS ? __ldcs(&seed[pid]) : seed[pid]; }
-    __device__ __forceinline__ void st_seed(uint32_t pid, uint2 v) const { if (RTX_STREAM_HINTS) __stcs(&seed[pid], v); else seed[pid] = v; }
+    __device__ __forceinline__ float4 ld(int plane, uint32_t pid) const { return __ldcs(&at(plane, pid)); }
+    __device__ __forceinline__ void stt(int plane, uint32_t pid, float4 v) const { __stcs(&at(plane, pid), v); }
+    __device__ __forceinline__ uint2 ld_seed(uint32_t pid) const { return __ldcs(&seed[pid]); }
+    __device__ __forceinline__ void st_seed(uint32_t pid, uint2 v) const { __stcs(&seed[pid], v); }
 };
 
 // queue entries and hit records a shading stage consumes (read once)
-template <typename T> __device__ __forceinline__ T ld_stream(const T* p) { return RTX_STREAM_HINTS ? __ldcs(p) : *p; }
+template <typename T> __device__ __forceinline__ T ld_stream(const T* p) { return __ldcs(p); }
 
 // Which paths a part (path range) of a pass owns: the contiguous range [p0, p0 + np), or — chunk != 0 — every parts-th chunk of `chunk`
 // consecutive paths (a few image rows), so that concurrent parts see the same mix of the image and finish together.  k = index in the part.

@@ -72,7 +72,6 @@ struct WaveBuffers {
     uint8_t* output = nullptr;         // gOutput slice 0
     rtx_camera_params* cam = nullptr;  // b0 (device copy)
     float* debug = nullptr;            // 64 floats
-    uint32_t* perm = nullptr; unsigned char* bin_keys = nullptr; uint32_t* bins = nullptr;   // RTX_FLAG_SORT_MATERIAL scratch
 };
 
 cudaError_t wave_alloc(WaveBuffers* B, uint32_t width, uint32_t height, uint32_t spp);
@@ -80,7 +79,7 @@ void wave_free(WaveBuffers* B);
 
 #define WAVE_MAX_EVENTS 96
 // stage kinds of rtx_last_pass_stage_ms (include/rtx_b200.h RTX_STAGE_*)
-enum StageKind { SK_GENERATE = 0, SK_CLOSEST, SK_ANY, SK_SHADE_PRIMARY, SK_DI_FINISH, SK_GI_STEP, SK_SCATTER, SK_FINALIZE, SK_ACCUMULATE, SK_SORT, SK_COUNT };
+enum StageKind { SK_GENERATE = 0, SK_CLOSEST, SK_ANY, SK_SHADE_PRIMARY, SK_DI_FINISH, SK_GI_STEP, SK_SCATTER, SK_FINALIZE, SK_ACCUMULATE, SK_COUNT };
 struct PassTiming {
     cudaEvent_t ev[WAVE_MAX_EVENTS] = {};   // [0],[1] bracket the pass; with stage_timing, ev[2+i] is recorded before launch i
     unsigned char kind[WAVE_MAX_EVENTS] = {};

@@ -302,16 +302,6 @@ def test_restir_frames_in_concurrent_parts(rtdx, orc):
         ctx.close()
 
 
-def test_material_sorted_queues_do_not_change_the_image(rtdx, orc):
-    """RTX_FLAG_SORT_MATERIAL bins every shading queue by hit material before k_gi_step; each path draws its own random numbers,
-    so the image, the reservoirs and the ray counts are bit-identical to the unsorted run (and to the oracle)."""
-    sc = rtdx.scenes.mesh_room(n=24)
-    ctx, gpu, cnt, ref, octr = _render_both(rtdx, orc, sc, 96, 64, 2, 6, rtdx.FLAG_SORT_MATERIAL)
-    assert cnt["closest_rays"] == octr["closest_rays"] and cnt["shadow_rays"] == octr["shadow_rays"], (cnt, octr)
-    assert (bits(gpu) != bits(ref)).sum() == 0
-    ctx.close()
-
-
 @pytest.mark.parametrize("scene_name", ["cornell", "mesh", "inst"])
 def test_legacy_rr_estimator_bit_exact(rtdx, orc, scene_name):
     """RTX_FLAG_LEGACY_RR (SURVEY 8f rank 4): the reference's older estimator (include/RayGen.hlsl + include/Hit.hlsl: RIS-10 NEE with one

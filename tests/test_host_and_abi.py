@@ -108,12 +108,16 @@ def test_abi_library_exports_every_declared_symbol(rtdx):
         assert hasattr(host, name)
 
 
-def test_python_constants_equal_the_header(rtdx):
-    """Every RTX_FLAG_* / RTX_OPT_* of include/rtx_b200.h has a Python constant of the same value (the bindings of tests and bench)."""
+def test_python_constants_are_exactly_the_header_flags_and_options(rtdx):
+    """include/rtx_b200.h defines exactly these RTX_FLAG_* / RTX_OPT_* names, and each has a Python constant of the same value (the
+    bindings of tests and bench)."""
     import re
     hdr = open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "include", "rtx_b200.h")).read()
     defs = dict((m.group(1), int(m.group(2), 0)) for m in re.finditer(r"#define\s+RTX_((?:FLAG|OPT)_\w+)\s+(0x[0-9a-fA-F]+|\d+)u", hdr))
-    assert len([k for k in defs if k.startswith("OPT_")]) >= 14 and len([k for k in defs if k.startswith("FLAG_")]) >= 6
+    assert sorted(defs) == sorted(["FLAG_JITTER", "FLAG_LAMBERT_ONLY", "FLAG_RESTIR", "FLAG_LEGACY_RR", "FLAG_FAST_MATH"] + [
+        "OPT_TRACE_STATS", "OPT_STAGE_TIMING", "OPT_PASS_PARTS", "OPT_TLAS_REBUILD", "OPT_TRACE_FETCH_TH", "OPT_TRACE_SCHED",
+        "OPT_TRACE_WAVES", "OPT_QUEUE_LPT", "OPT_TRACE_CTAS", "OPT_PASS_GRAPH", "OPT_SHADOW_OVERLAP", "OPT_PART_ROWS",
+        "OPT_PASS_PIPELINE", "OPT_FRAME_PIPELINE"])
     for name, value in defs.items():
         assert getattr(rtdx, name) == value, name
 
@@ -152,6 +156,19 @@ def test_create_validates_the_path_length_before_touching_a_device(rtdx):
             assert st != 1, lib.rtx_last_error()             # passes the argument check (fails later only for want of a GPU)
         else:
             assert st == 1 and b"bounces" in lib.rtx_last_error()
+
+
+@pytest.mark.parametrize("flag", [4, 64])
+def test_create_rejects_unknown_flags_before_touching_a_device(rtdx, flag):
+    """A flag bit the engine does not know (4 selected the removed material-binned queues) fails with RTX_ERR_ARG and an error that
+    names the valid flags, instead of rendering in some other mode."""
+    lib = rtdx.load_library()
+    cfg = rtdx.RtxConfig(C.sizeof(rtdx.RtxConfig), 0, 16, 16, 3, 4, 4, rtdx.FLAG_JITTER | flag, 1, None)
+    h = C.c_void_p()
+    st = lib.rtx_create(C.byref(cfg), C.byref(h))
+    if h:
+        lib.rtx_destroy(h)
+    assert st == 1 and b"unknown flags" in lib.rtx_last_error() and b"RTX_FLAG_FAST_MATH" in lib.rtx_last_error()
 
 
 def test_engine_free_host_library_has_no_cuda_dependency(rtdx):
