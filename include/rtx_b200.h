@@ -97,6 +97,30 @@ void       rtx_destroy(rtx_ctx*);
 rtx_status rtx_upload_model(rtx_ctx*, const rtx_vertex* v, uint32_t n_vertices, const uint32_t* indices, uint32_t n_indices,
                             uint32_t material_id_offset, uint32_t* model_id_out);
 rtx_status rtx_blas_info_get(rtx_ctx*, uint32_t model_id, rtx_blas_info* out);
+/* Deforming meshes (DXR: a BLAS built with ALLOW_UPDATE, then PERFORM_UPDATE): new vertex data for an uploaded model — same vertex
+ * count, same index buffer, same material_id_offset (topology changes go through rtx_upload_model).  Both modes update everything
+ * derived from the vertices: the model's vertex buffer in place, its triangle records, its node boxes or a new BVH, its closest-hit
+ * attribute records, its object-space bounds in the per-model tables, the world boxes of its instances and the TLAS (one-node rewrite,
+ * refit or rebuild as rtx_set_instances chooses, over the instance list already set; without instances only the model is updated).
+ * Leaf boxes are padded as the builder pads them (2^-15 of the largest absolute coordinate of the NEW bounds), so hits stay those of
+ * the brute-force definition in both modes.
+ * Stream order: like every entry point, ordered after all passes already queued (pipelined ones included); work queued after the call
+ * sees the new geometry, captured pass graphs included (no recapture).  The call does not reset the accumulation (only a view change
+ * does) and does not touch the emissive-triangle list: a caller that deforms an emissive model collects and sets it again.
+ * Errors: RTX_ERR_ARG before any device work for a null context, an unknown model, a vertex count that differs from the upload, an
+ * unknown mode, a null pointer with a nonzero count, and (_device) memory that is not device or managed memory of cfg.device.
+ * RTX_UPDATE_REBUILD re-runs the traversal-stack depth check of rtx_set_instances and returns RTX_ERR_STATE as it does. */
+#define RTX_UPDATE_REFIT   0u  /* keep the BVH topology, recompute every node box bottom-up (DXR PERFORM_UPDATE).  Child order stays that of
+                                * the build: after a large deformation traversal gets slower, not wrong (RTX_UPDATE_REBUILD restores it) */
+#define RTX_UPDATE_REBUILD 1u  /* full build over the new positions into new buffers, swapped in for the old ones (restores tree quality);
+                                * the old buffers are freed once the stream has passed every user; synchronises the host */
+/* from host memory (the call may synchronise the host, like rtx_upload_model) */
+rtx_status rtx_update_model(rtx_ctx*, uint32_t model_id, const rtx_vertex* v, uint32_t n_vertices, uint32_t mode);
+/* from a device buffer of n_vertices * 28 bytes on the context's device, copied on the context stream.  With RTX_UPDATE_REFIT the call
+ * neither synchronises the host nor allocates: the per-frame path of an animated mesh.  The bounds the refit computes are copied back
+ * behind an event and read before their next host use (rtx_set_instances, rtx_upload_model's table rebuild, rtx_blas_info_get), which
+ * then waits for the refit. */
+rtx_status rtx_update_model_device(rtx_ctx*, uint32_t model_id, const void* d_vertices, uint32_t n_vertices, uint32_t mode);
 /* binding t4 (rdn/Renderer.cpp:1274-1282) and t5 */
 rtx_status rtx_set_material_ids(rtx_ctx*, const uint32_t* ids, uint32_t n);
 rtx_status rtx_set_materials(rtx_ctx*, const rtx_material* m, uint32_t n);

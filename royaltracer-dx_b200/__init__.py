@@ -36,6 +36,7 @@ assert camera_dt.itemsize == 512 and desc_dt.itemsize == 64 and ray_dt.itemsize 
 
 FLAG_JITTER, FLAG_LAMBERT_ONLY, FLAG_RESTIR, FLAG_LEGACY_RR, FLAG_FAST_MATH = 1, 2, 8, 16, 32
 OPT_TRACE_STATS, OPT_STAGE_TIMING, OPT_PASS_PARTS, OPT_TLAS_REBUILD, OPT_TRACE_FETCH_TH, OPT_TRACE_SCHED, OPT_TRACE_WAVES, OPT_QUEUE_LPT, OPT_TRACE_CTAS, OPT_PASS_GRAPH, OPT_SHADOW_OVERLAP, OPT_PART_ROWS, OPT_PASS_PIPELINE, OPT_FRAME_PIPELINE = 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 14
+UPDATE_REFIT, UPDATE_REBUILD = 0, 1       # rtx_update_model* modes (include/rtx_b200.h)
 MISS = 0xFFFFFFFF
 STAGE_NAMES = ["generate", "closest", "any", "shade_primary", "di_finish", "gi_step", "scatter", "finalize", "accumulate"]
 
@@ -57,7 +58,8 @@ class RtxBlasInfo(C.Structure):
 
 
 # every symbol include/rtx_b200.h declares (tests check the library exports all of them)
-ABI_SYMBOLS = ["rtx_last_error", "rtx_create", "rtx_destroy", "rtx_upload_model", "rtx_blas_info_get", "rtx_set_material_ids",
+ABI_SYMBOLS = ["rtx_last_error", "rtx_create", "rtx_destroy", "rtx_upload_model", "rtx_update_model", "rtx_update_model_device",
+               "rtx_blas_info_get", "rtx_set_material_ids",
                "rtx_set_materials", "rtx_set_instances", "rtx_set_emissive_triangles", "rtx_set_camera", "rtx_render_pass",
                "rtx_reset_accum", "rtx_synchronize", "rtx_read_accum", "rtx_read_output", "rtx_read_output_async", "rtx_wait_output", "rtx_set_resolve_source",
                "rtx_accum_device_ptr", "rtx_trace",
@@ -89,6 +91,8 @@ def load_library():
     lib.rtx_destroy.argtypes = [vp]
     lib.rtx_destroy.restype = None
     lib.rtx_upload_model.argtypes = [vp, vp, u32, vp, u32, u32, C.POINTER(u32)]
+    lib.rtx_update_model.argtypes = [vp, u32, vp, u32, u32]
+    lib.rtx_update_model_device.argtypes = [vp, u32, vp, u32, u32]
     lib.rtx_blas_info_get.argtypes = [vp, u32, C.POINTER(RtxBlasInfo)]
     lib.rtx_set_material_ids.argtypes = [vp, vp, u32]
     lib.rtx_set_materials.argtypes = [vp, vp, u32]
@@ -262,6 +266,19 @@ class Context:
         mid = C.c_uint32()
         self._check(self.lib.rtx_upload_model(self.handle, _ptr(v), v.size, _ptr(i), i.size, material_id_offset, C.byref(mid)))
         return mid.value
+
+    def update_model(self, model_id, vertices, mode=UPDATE_REFIT):
+        """New positions / normals for an uploaded model (same vertex count and indices): refit (default) or rebuild its BVH; instance
+        boxes and the TLAS follow.  The accumulation is not reset and the light list is not touched."""
+        v = np.ascontiguousarray(vertices, dtype=vertex_dt)
+        self._check(self.lib.rtx_update_model(self.handle, model_id, _ptr(v), v.size, mode))
+
+    def update_model_device(self, model_id, buf, n_vertices, mode=UPDATE_REFIT):
+        """The same from device memory of n_vertices * 28 bytes: an int device pointer or anything with data_ptr() (a torch tensor),
+        copied on the context stream; with UPDATE_REFIT the call neither waits nor allocates.  Work that wrote the buffer on another
+        stream must be complete, or ordered before the context stream, when the call is made."""
+        ptr = buf.data_ptr() if hasattr(buf, "data_ptr") else buf
+        self._check(self.lib.rtx_update_model_device(self.handle, model_id, C.c_void_p(int(ptr) if ptr else None), n_vertices, mode))
 
     def blas_info(self, model_id):
         info = RtxBlasInfo()

@@ -53,6 +53,13 @@ __device__ __host__ __forceinline__ float dec_f(unsigned int e) {
 #endif
 }
 
+// the padding of every primitive box: 2^-15 of the largest absolute coordinate of the reduced bounds
+__device__ __forceinline__ float leaf_pad(const BuildCounters* c) {
+    float s = 0.0f;
+    for (int k = 0; k < 6; k++) s = fmaxf(s, fabsf(dec_f(c->bounds[k])));
+    return s * 3.0517578125e-5f + 1e-30f;
+}
+
 __global__ void k_init_counters(BuildCounters* c) {
     c->nodes = 1; c->prims = 0; c->tasks_out = 0; c->hier_nodes = 0;
     c->bounds[0] = c->bounds[1] = c->bounds[2] = 0xffffffffu;
@@ -159,9 +166,7 @@ __global__ void k_leaf_boxes(const float4* __restrict__ plo, const float4* __res
                              float4* __restrict__ nlo, float4* __restrict__ nhi, int* __restrict__ clusters, const BuildCounters* c) {
     int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= n) return;
-    float s = 0.0f;
-    for (int k = 0; k < 6; k++) s = fmaxf(s, fabsf(dec_f(c->bounds[k])));
-    const float pad = s * 3.0517578125e-5f + 1e-30f;
+    const float pad = leaf_pad(c);
     const uint32_t p = vals[j];
     float4 l = plo[p], h = phi[p];
     nlo[j] = make_float4(l.x - pad, l.y - pad, l.z - pad, 0.0f);
@@ -426,9 +431,7 @@ template <int PRIM_F4, typename Source>
 __global__ void k_single_node(Source src, const float4* __restrict__ plo, const float4* __restrict__ phi, int n, uint4* out_nodes,
                               float4* out_prims, BuildCounters* c) {
     if (threadIdx.x || blockIdx.x) return;
-    float s = 0.0f;
-    for (int k = 0; k < 6; k++) s = fmaxf(s, fabsf(dec_f(c->bounds[k])));
-    const float pad = s * 3.0517578125e-5f + 1e-30f;
+    const float pad = leaf_pad(c);
     float l[3] = {INFINITY, INFINITY, INFINITY}, h[3] = {-INFINITY, -INFINITY, -INFINITY};
     for (int i = 0; i < n; i++) {
         const float4 a = plo[i], b = phi[i];
@@ -634,10 +637,31 @@ __device__ __forceinline__ void node_box(const uint4* np, float lo[3], float hi[
     }
 }
 
-// one thread per node of one level: child boxes from the refitted children (inner) or the instances' world boxes (leaves), then the same
-// origin / exponent / outward quantisation as emit_node
-__global__ void k_refit_level(uint4* __restrict__ nodes, uint32_t first, uint32_t count, const float4* __restrict__ prims,
-                              const float4* __restrict__ box_lo, const float4* __restrict__ box_hi) {
+// Leaf-box sources of the refit: the box of the primitive record in leaf slot `slot`, folded into l / h.
+struct InstLeafBoxes {   // TLAS: the instance's (already padded) world box, found through the instance id in .w.y of the record
+    const float4* prims; const float4* box_lo; const float4* box_hi;
+    __device__ __forceinline__ void fold(uint32_t slot, float l[3], float h[3]) const {
+        const uint32_t inst = __float_as_uint(prims[4 * (size_t)slot + 3].y);
+        const float4 a = box_lo[inst], b = box_hi[inst];
+        l[0] = fminf(l[0], a.x); l[1] = fminf(l[1], a.y); l[2] = fminf(l[2], a.z);
+        h[0] = fmaxf(h[0], b.x); h[1] = fmaxf(h[1], b.y); h[2] = fmaxf(h[2], b.z);
+    }
+};
+struct TriLeafBoxes {    // BLAS: the refitted triangle record, padded as k_tri_boxes + k_leaf_boxes / k_single_node pad a triangle
+    const float4* prims; const BuildCounters* ctr;
+    __device__ __forceinline__ void fold(uint32_t slot, float l[3], float h[3]) const {
+        const float pad = leaf_pad(ctr);
+        const float4 a = prims[3 * (size_t)slot], b = prims[3 * (size_t)slot + 1], d = prims[3 * (size_t)slot + 2];
+        l[0] = fminf(l[0], fminf(a.x, fminf(b.x, d.x)) - pad); h[0] = fmaxf(h[0], fmaxf(a.x, fmaxf(b.x, d.x)) + pad);
+        l[1] = fminf(l[1], fminf(a.y, fminf(b.y, d.y)) - pad); h[1] = fmaxf(h[1], fmaxf(a.y, fmaxf(b.y, d.y)) + pad);
+        l[2] = fminf(l[2], fminf(a.z, fminf(b.z, d.z)) - pad); h[2] = fmaxf(h[2], fmaxf(a.z, fmaxf(b.z, d.z)) + pad);
+    }
+};
+
+// one thread per node of one level: child boxes from the refitted children (inner) or the leaf source (leaves), then the same
+// origin / exponent / outward quantisation as emit_node.  Topology, child order and primitive order stay those of the build.
+template <typename Leaves>
+__global__ void k_refit_level(uint4* __restrict__ nodes, uint32_t first, uint32_t count, Leaves leaves) {
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= count) return;
     uint4* np = nodes + (size_t)(first + t) * 5;
@@ -656,11 +680,7 @@ __global__ void k_refit_level(uint4* __restrict__ nodes, uint32_t first, uint32_
             for (int a = 0; a < 3; a++) { clo[s][a] = INFINITY; chi[s][a] = -INFINITY; }
             for (int k = 0; k < 3; k++) {
                 if (!((W >> (3 * s + k)) & 1u)) continue;
-                const uint32_t slot = n1.y + __popc(W & ((1u << (3 * s + k)) - 1u));
-                const uint32_t inst = __float_as_uint(prims[4 * (size_t)slot + 3].y);
-                const float4 l = box_lo[inst], h = box_hi[inst];
-                clo[s][0] = fminf(clo[s][0], l.x); clo[s][1] = fminf(clo[s][1], l.y); clo[s][2] = fminf(clo[s][2], l.z);
-                chi[s][0] = fmaxf(chi[s][0], h.x); chi[s][1] = fmaxf(chi[s][1], h.y); chi[s][2] = fmaxf(chi[s][2], h.z);
+                leaves.fold(n1.y + __popc(W & ((1u << (3 * s + k)) - 1u)), clo[s], chi[s]);
             }
             used[s] = true;
         }
@@ -689,15 +709,66 @@ __global__ void k_refit_level(uint4* __restrict__ nodes, uint32_t first, uint32_
     np[4] = make_uint4(pack4(qhi[1]), pack4(qhi[1] + 4), pack4(qhi[2]), pack4(qhi[2] + 4));
 }
 
+// one launch per level, deepest first: a node reads the boxes of its inner children, refitted by the launch before
+template <typename Leaves>
+static cudaError_t refit_levels(Bvh8* b, Leaves leaves, cudaStream_t stream) {
+    for (int lv = (int)b->n_levels - 1; lv >= 0; lv--) {
+        const uint32_t first = b->level_start[lv], count = b->level_start[lv + 1] - first;
+        if (count) k_refit_level<Leaves><<<(count + 127) / 128, 128, 0, stream>>>(b->nodes, first, count, leaves);
+    }
+    return cudaGetLastError();
+}
+
 cudaError_t refit_tlas(const float4* d_inst_recs, const float4* d_box_lo, const float4* d_box_hi, uint32_t n_instances, Bvh8* b,
                        cudaStream_t stream) {
     if (!b->nodes || !b->prims || b->n_prims != n_instances || b->n_levels == 0u || b->level_start[b->n_levels] != b->n_nodes)
         return cudaErrorInvalidValue;
     k_refit_prims<<<(n_instances + 255) / 256, 256, 0, stream>>>(d_inst_recs, n_instances, b->prims);
-    for (int lv = (int)b->n_levels - 1; lv >= 0; lv--) {
-        const uint32_t first = b->level_start[lv], count = b->level_start[lv + 1] - first;
-        if (count) k_refit_level<<<(count + 127) / 128, 128, 0, stream>>>(b->nodes, first, count, b->prims, d_box_lo, d_box_hi);
+    return refit_levels(b, InstLeafBoxes{b->prims, d_box_lo, d_box_hi}, stream);
+}
+
+// ---- BLAS refit (DXR PERFORM_UPDATE) ---------------------------------------------------------------------------------
+// leaf order of the triangle records: prims[3k] carries its primitive id in .w (TriSource::write).  Rewrites each record from the new
+// vertices and folds its box into the model bounds (the reduction of k_tri_boxes: the padding of the level pass needs them).
+__global__ void k_refit_tris(const uint8_t* __restrict__ verts, const uint32_t* __restrict__ idx, uint32_t n, float4* __restrict__ prims,
+                             BuildCounters* c) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool valid = k < n;
+    float lx = 0, ly = 0, lz = 0, hx = 0, hy = 0, hz = 0;
+    if (valid) {
+        float4* r = prims + 3 * (size_t)k;
+        TriSource{verts, idx}.write(r, __float_as_uint(r[0].w));
+        const float4 a = r[0], b = r[1], d = r[2];
+        lx = fminf(a.x, fminf(b.x, d.x)); hx = fmaxf(a.x, fmaxf(b.x, d.x));
+        ly = fminf(a.y, fminf(b.y, d.y)); hy = fmaxf(a.y, fmaxf(b.y, d.y));
+        lz = fminf(a.z, fminf(b.z, d.z)); hz = fmaxf(a.z, fmaxf(b.z, d.z));
     }
+    reduce_bounds(c, lx, ly, lz, hx, hy, hz, valid);
+}
+
+// the padded model bounds (build_generic's out->lo / hi) into the model's table entries, when they exist, and into out6
+__global__ void k_refit_tables(const BuildCounters* c, BlasRef* ref, BlasBounds* bb, float* out6) {
+    const float pad = leaf_pad(c);
+    for (int k = 0; k < 3; k++) {
+        const float l = dec_f(c->bounds[k]) - pad, h = dec_f(c->bounds[3 + k]) + pad;
+        out6[k] = l; out6[3 + k] = h;
+        if (ref) { ref->lo[k] = l; ref->hi[k] = h; }
+        if (bb) { bb->lo[k] = l; bb->hi[k] = h; }
+    }
+}
+
+cudaError_t refit_blas(const uint8_t* d_vertices, const uint32_t* d_indices, uint32_t n_tris, Bvh8* b, void* d_scratch, BlasRef* d_ref,
+                       BlasBounds* d_bounds, float* d_out6, cudaStream_t stream) {
+    static_assert(sizeof(BuildCounters) <= 256, "refit_blas: scratch too small");
+    if (!b->nodes || !b->prims || b->n_prims != n_tris || b->n_levels == 0u || b->level_start[b->n_levels] != b->n_nodes)
+        return cudaErrorInvalidValue;
+    if (n_tris == 0) return cudaSuccess;
+    BuildCounters* ctr = (BuildCounters*)d_scratch;
+    k_init_counters<<<1, 1, 0, stream>>>(ctr);
+    k_refit_tris<<<(n_tris + 255) / 256, 256, 0, stream>>>(d_vertices, d_indices, n_tris, b->prims, ctr);
+    const cudaError_t e = refit_levels(b, TriLeafBoxes{b->prims, ctr}, stream);
+    if (e != cudaSuccess) return e;
+    k_refit_tables<<<1, 1, 0, stream>>>(ctr, d_ref, d_bounds, d_out6);
     return cudaGetLastError();
 }
 

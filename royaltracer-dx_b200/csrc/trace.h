@@ -51,4 +51,12 @@ cudaError_t launch_instance_records(const rtx_instance_desc* d_descs, const rtx_
                                     uint32_t n, float4* d_recs, float4* d_lo, float4* d_hi, unsigned int* d_scratch6 /* 6 words per instance */,
                                     cudaStream_t stream);
 
+// BLAS REFIT over new vertex positions (DXR PERFORM_UPDATE; same vertex count and index buffer as the build): keeps the topology, child
+// order and leaf order of the build, rewrites the triangle records from the vertices and recomputes every node bottom-up, one launch per
+// level, with the builder's padding (2^-15 of the NEW bounds) and outward quantisation.  The padded model bounds go to inout's table
+// entries d_ref / d_bounds (when non-null) and to d_out6 (6 floats, device).  inout->lo / hi are NOT updated (the host copy is the
+// caller's: it copies d_out6 back).  Stream-ordered, no allocation, no host synchronisation.  d_scratch = 256 B of device scratch.
+cudaError_t refit_blas(const uint8_t* d_vertices, const uint32_t* d_indices, uint32_t n_tris, Bvh8* inout, void* d_scratch, BlasRef* d_ref,
+                       BlasBounds* d_bounds, float* d_out6, cudaStream_t stream);
+
 }  // namespace rtx

@@ -309,3 +309,35 @@ def camera_rays(cam, width, height, step=1):
     rays["origin"] = viewI[:3, 3]; rays["direction"] = d.astype(np.float32)
     rays["tmin"] = 1e-4; rays["tmax"] = 1e4
     return rays
+
+
+def deform(vertices, t, amplitude, seed=0):
+    """A seeded, deterministic deformation of a model's vertex array (vertex_dt) for animated-mesh workloads: a travelling wave along
+    the vertex normals (amplitude x the model's extent, phase moving with t) plus a twist about a seeded axis through the centre of the
+    bounds (amplitude x 1 rad across the extent).  Returns a new float32 vertex_dt array; normals are rotated by the twist, the material
+    word is kept.  Vertices without a normal are only twisted."""
+    v = np.ascontiguousarray(vertices, dtype=vertex_dt)
+    p = v["position"].astype(np.float64)
+    n = v["normal_material"][:, :3].astype(np.float64)
+    out = v.copy()
+    if p.shape[0] == 0:
+        return out
+    rng = np.random.RandomState(seed)
+    k = rng.normal(size=3); k /= np.linalg.norm(k)
+    axis = rng.normal(size=3); axis /= np.linalg.norm(axis)
+    lo, hi = p.min(axis=0), p.max(axis=0)
+    c = 0.5 * (lo + hi)
+    size = float((hi - lo).max()) or 1.0
+    freq = 2.0 * np.pi * (1.0 + rng.rand()) / size
+    phase = 2.0 * np.pi * rng.rand()
+    q = p - c
+    q = q + n * (amplitude * size * 0.1 * np.sin(freq * (q @ k) - 2.0 * np.pi * t + phase))[:, None]
+    ang = amplitude * (q @ axis) / size                     # Rodrigues' rotation about `axis`, angle varying along it
+    cs, sn = np.cos(ang)[:, None], np.sin(ang)[:, None]
+
+    def rot(x):
+        return x * cs + np.cross(axis, x) * sn + axis * (x @ axis)[:, None] * (1.0 - cs)
+
+    out["position"] = (rot(q) + c).astype(np.float32)
+    out["normal_material"][:, :3] = rot(n).astype(np.float32)
+    return out
