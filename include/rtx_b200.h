@@ -196,24 +196,18 @@ rtx_status rtx_last_pass_stage_ms(rtx_ctx*, float* ms_by_stage, uint32_t n_stage
 /* runtime options.  RTX_OPT_TRACE_STATS: closest-hit traversals of rtx_render_pass also count nodes/triangles/instances
  * (instrumented kernel variant: for the roofline's B_ray, never for timed runs), and the shading stages count the paths they
  * replay with guarded IEEE operations (rtx_counters.shading_replays).  RTX_OPT_STAGE_TIMING: record CUDA events
- * around every traversal launch of a pass so that rtx_last_pass_ms can report the traversal share.
+ * around every traversal launch of a pass so that rtx_last_pass_ms can report the traversal share.  Either one also traces a
+ * pass's DI visibility rays in sequence rather than on a side stream.
  * RTX_OPT_PASS_PARTS: 1..4 path ranges of a pass that run concurrently on separate CUDA streams (default 2; the image
- * does not depend on it; passes with per-launch events, statistics or ReSTIR reuse always run as one part). */
+ * does not depend on it; passes with per-launch events, statistics or ReSTIR reuse always run as one part).
+ * The traversal launch shape, the trace order and the row interleave of the path ranges are fixed at their measured optima
+ * (csrc/trace.cu, csrc/wavefront.cu).  Values 5..9, 11 and 12 are retired and not reused: rtx_set_option rejects them as unknown. */
 #define RTX_OPT_TRACE_STATS   1u
 #define RTX_OPT_STAGE_TIMING  2u
 #define RTX_OPT_PASS_PARTS    3u
 #define RTX_OPT_TLAS_REBUILD  4u   /* 1: rtx_set_instances always rebuilds the TLAS; 0 (default): it refits the last build when the instance
                                     * list still names the same models (rdn/Renderer.cpp:594 refits every frame) */
-/* launch tuning of the traversal kernels (0 = built-in default, the measured optimum; csrc/trace.cu): */
-#define RTX_OPT_TRACE_FETCH_TH 5u  /* a warp refills its idle lanes when fewer than this many lanes are still traversing (default 24) */
-#define RTX_OPT_TRACE_SCHED    6u  /* phase scheduling thresholds th_tri | th_inst << 8 | th_node << 16 (default 0x060808) */
-#define RTX_OPT_TRACE_WAVES    7u  /* persistent grid = SMs x resident CTAs x waves (default 1) */
-#define RTX_OPT_QUEUE_LPT       8u  /* 1 (default): closest-hit queues are traced longest-processing-time-first (rays that cross the bounds of the
-                                    * scene's large instances before the others); 0: in emission order.  The image does not depend on it. */
-#define RTX_OPT_TRACE_CTAS      9u  /* resident CTAs per SM of the persistent traversal grid (0 = default: all the register budget allows) */
 #define RTX_OPT_PASS_GRAPH     10u  /* 1 (default): a pass of a static configuration is captured once into a CUDA graph and replayed; 0: plain launches */
-#define RTX_OPT_SHADOW_OVERLAP 11u  /* 1 (default): the DI visibility rays of a pass are traced on a side stream beside the indirect bounces; 0: in sequence */
-#define RTX_OPT_PART_ROWS      12u  /* concurrent path ranges own interleaved chunks of this many image rows: 0 = contiguous ranges, 1..64, 0xffffffff (default) = chosen per frame size */
 #define RTX_OPT_PASS_PIPELINE  13u  /* 1 (default): rtx_render_pass calls that directly follow each other overlap (two sets of pass buffers, accumulation in call order: bit-identical); 0: one pass at a time */
 #define RTX_OPT_FRAME_PIPELINE 14u  /* 1 (default): a per-frame loop rtx_set_instances (<= 8 instances, same models) -> rtx_set_camera -> rtx_render_pass -> rtx_read_output_async keeps two sets of per-frame state and overlaps consecutive frames (bit-identical); 0: one frame at a time */
 rtx_status rtx_set_option(rtx_ctx*, uint32_t option, uint32_t value);

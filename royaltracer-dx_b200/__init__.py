@@ -35,7 +35,7 @@ assert vertex_dt.itemsize == 28 and material_dt.itemsize == 128 and props_dt.ite
 assert camera_dt.itemsize == 512 and desc_dt.itemsize == 64 and ray_dt.itemsize == 32 and hit_dt.itemsize == 20
 
 FLAG_JITTER, FLAG_LAMBERT_ONLY, FLAG_RESTIR, FLAG_LEGACY_RR, FLAG_FAST_MATH = 1, 2, 8, 16, 32
-OPT_TRACE_STATS, OPT_STAGE_TIMING, OPT_PASS_PARTS, OPT_TLAS_REBUILD, OPT_TRACE_FETCH_TH, OPT_TRACE_SCHED, OPT_TRACE_WAVES, OPT_QUEUE_LPT, OPT_TRACE_CTAS, OPT_PASS_GRAPH, OPT_SHADOW_OVERLAP, OPT_PART_ROWS, OPT_PASS_PIPELINE, OPT_FRAME_PIPELINE = 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 14
+OPT_TRACE_STATS, OPT_STAGE_TIMING, OPT_PASS_PARTS, OPT_TLAS_REBUILD, OPT_PASS_GRAPH, OPT_PASS_PIPELINE, OPT_FRAME_PIPELINE = 1, 2, 3, 4, 10, 13, 14
 UPDATE_REFIT, UPDATE_REBUILD = 0, 1       # rtx_update_model* modes (include/rtx_b200.h)
 MISS = 0xFFFFFFFF
 STAGE_NAMES = ["generate", "closest", "any", "shade_primary", "di_finish", "gi_step", "scatter", "finalize", "accumulate"]

@@ -65,12 +65,12 @@ struct rtx_ctx {
     unsigned int* h_overflow = nullptr;     // pinned copy written behind every asynchronous read-back (rtx_wait_output looks at it)
     void* d_trace_rays = nullptr; size_t cap_trace_rays = 0; void* d_trace_hits = nullptr; size_t cap_trace_hits = 0;   // rtx_trace staging
     size_t cap_material_ids = 0, cap_materials = 0, cap_lights = 0;
-    int num_sms = 148, fetch_th = 0, sched = 0, waves = 0, ctas_per_sm = 0;     // traversal launch tuning (0 = the built-in defaults, trace.cu)
+    int num_sms = 148;
     // multi-GPU (rtx_comm_init): one NCCL reduce of gPermanentData per progressive pass, on the side stream (SURVEY.md 8e)
     void* comm = nullptr; int comm_rank = 0, comm_world = 1;
     float4* d_total = nullptr;              // root only: the sum over ranks; rtx_read_output* resolve it
     cudaEvent_t ev_pass = nullptr, ev_reduced = nullptr;
-    float heavy_lo[3] = {0, 0, 0}, heavy_hi[3] = {0, 0, 0}; bool heavy_valid = false, lpt = true;   // SceneData::heavy_* (queue order only)
+    float heavy_lo[3] = {0, 0, 0}, heavy_hi[3] = {0, 0, 0}; bool heavy_valid = false;   // SceneData::heavy_* (queue order only)
     uint64_t launches = 0;
     PassTiming timing;
     bool trace_stats = false;
@@ -670,7 +670,7 @@ static SceneData scene_data(rtx_ctx* c, int set = 0) {
     S.cfg_flags = c->cfg.flags; S.bounces = c->cfg.bounces; S.nee_samples = c->cfg.nee_samples; S.nee_samples_di = c->cfg.nee_samples_di;
     S.width = c->cfg.width; S.height = c->cfg.height;
     for (int r = 0; r < 3; r++) { S.heavy_lo[r] = c->heavy_lo[r]; S.heavy_hi[r] = c->heavy_hi[r]; }
-    S.heavy_valid = c->heavy_valid && c->lpt ? 1u : 0u;
+    S.heavy_valid = c->heavy_valid;
     return S;
 }
 
@@ -681,7 +681,7 @@ static SceneAS make_as(rtx_ctx* c, int set = 0) {
     a.tlas_nodes = tl.nodes; a.inst_recs = tl.prims; a.blas = c->d_blas; a.n_instances = c->n_instances;
     a.one_bits = 0x3F800000u;
     a.overflow = c->d_overflow;
-    a.num_sms = c->num_sms; a.fetch_th = c->fetch_th; a.sched = c->sched; a.waves = c->waves; a.ctas_per_sm = c->ctas_per_sm;
+    a.num_sms = c->num_sms;
     return a;
 }
 
@@ -764,7 +764,6 @@ extern "C" rtx_status rtx_render_pass(rtx_ctx* c, uint32_t first_sample, uint32_
             RTX_CK(cudaStreamWaitEvent(st_, c->ev_state, 0));
             RTX_CK(cudaStreamWaitEvent(st_, c->ev_acc[lane], 0));           // the previous pass in these buffers (it may have run on the caller's stream)
             if (lane) {
-                B.shadow_overlap = c->wb.shadow_overlap; B.part_rows = c->wb.part_rows;
                 if (!c->wb.use_graph) B.use_graph = false;
                 T.stage_timing = false; T.stats = nullptr;
             }
@@ -1237,16 +1236,9 @@ extern "C" rtx_status rtx_set_option(rtx_ctx* c, uint32_t option, uint32_t value
         if (value < 1u || value > (uint32_t)WAVE_MAX_PARTS) return fail(RTX_ERR_ARG, "rtx_set_option: RTX_OPT_PASS_PARTS must be 1..4");
         c->wb.parts = (int)value;
     }
-    else if (option == RTX_OPT_TRACE_FETCH_TH) { if (value > 32u) return fail(RTX_ERR_ARG, "rtx_set_option: RTX_OPT_TRACE_FETCH_TH must be 0..32"); c->fetch_th = (int)value; }
-    else if (option == RTX_OPT_TRACE_SCHED) c->sched = (int)(value & 0xffffffu);
-    else if (option == RTX_OPT_TRACE_WAVES) { if (value > 8u) return fail(RTX_ERR_ARG, "rtx_set_option: RTX_OPT_TRACE_WAVES must be 0..8"); c->waves = (int)value; }
-    else if (option == RTX_OPT_QUEUE_LPT) c->lpt = value != 0;
     else if (option == RTX_OPT_PASS_GRAPH) { c->wb.use_graph = value != 0; c->wb2.use_graph = value != 0; }
-    else if (option == RTX_OPT_SHADOW_OVERLAP) c->wb.shadow_overlap = value != 0;
     else if (option == RTX_OPT_PASS_PIPELINE) c->pipeline = value != 0;
     else if (option == RTX_OPT_FRAME_PIPELINE) c->frame_pipeline = value != 0;
-    else if (option == RTX_OPT_PART_ROWS) { if (value > 64u && value != 0xffffffffu) return fail(RTX_ERR_ARG, "rtx_set_option: RTX_OPT_PART_ROWS must be 0..64 or 0xffffffff (automatic)"); c->wb.part_rows = value == 0xffffffffu ? -1 : (int)value; }
-    else if (option == RTX_OPT_TRACE_CTAS) { if (value > 32u) return fail(RTX_ERR_ARG, "rtx_set_option: RTX_OPT_TRACE_CTAS must be 0..32"); c->ctas_per_sm = (int)value; }
     else return fail(RTX_ERR_ARG, "rtx_set_option: unknown option");
     return RTX_OK;
 }

@@ -56,12 +56,7 @@ struct SceneAS {
                           // selector as an immediate (with the constant folded in, ptxas re-materialised a selector register per PRMT: 43 extra
                           // IMAD.U32 per node test)
     unsigned int* overflow;   // per-context word raised when a traversal stack overflows (checked and cleared by the API, api.cu check_overflow)
-    // launch tuning of the traversal kernels (rtx_set_option RTX_OPT_TRACE_*; defaults = the measured optimum, trace.cu)
-    int num_sms;          // of the context's device
-    int fetch_th;         // refill the warp's idle lanes when fewer than this many lanes are still traversing
-    int sched;            // th_tri | th_inst << 8 | th_node << 16 (phase scheduling, traverse.cuh)
-    int waves;            // persistent grid = num_sms * resident CTAs * waves
-    int ctas_per_sm;      // resident CTAs per SM the persistent grid uses (0 = all the register budget allows)
+    int num_sms;          // of the context's device: sizes the persistent traversal grid (trace.cu launch_trace)
 };
 
 // Ray queue entry layout (SoA): o_tmin[j] = (o.xyz, tmin), d_tmax[j] = (d.xyz, tmax).

@@ -7,7 +7,6 @@
 // memory latency — see DESIGN.md §Kernels).
 #include <algorithm>
 using std::max;
-using std::min;
 
 #include "trace.h"
 #include "traverse.cuh"
@@ -186,11 +185,11 @@ cudaError_t launch_trace(const SceneAS& S, const float4* o_tmin, const float4* d
     // `cursor` = two words, both 0 between launches: [0] the ray cursor, [1] the count of finished CTAs; the last CTA of a launch
     // resets [0] (and atomicInc wraps [1]), so no memset precedes the launch.
     const int sms = S.num_sms > 0 ? S.num_sms : 148;
-    const int fetch_th = S.fetch_th > 0 ? S.fetch_th : FETCH_THRESHOLD, sched = S.sched ? S.sched : RTX_SCHED_DEFAULT, waves = S.waves > 0 ? S.waves : 1;
-    // persistent: the resident CTAs of the machine (x waves), or this launch's share of them when several traversals run concurrently
+    // persistent: the resident CTAs of the machine, or this launch's share of them when several traversals run concurrently
     // (wave_render_pass: the parts' kernels are then co-resident and one part's drain phase overlaps the other's work)
-    const int ctas = S.ctas_per_sm > 0 ? min(S.ctas_per_sm, RTX_TRACE_MINB) : RTX_TRACE_MINB;
-    const int grid = max(sms, sms * ctas * waves / max(grid_share, 1));
+    const int grid = max(sms, sms * RTX_TRACE_MINB / max(grid_share, 1));
+    // (run-time kernel arguments on purpose: folded into compile-time constants they reschedule most of trace_kernel's SASS)
+    const int fetch_th = FETCH_THRESHOLD, sched = RTX_SCHED_DEFAULT;
     if (stats) {
         if (any_hit) trace_kernel<true, true><<<grid, TRACE_BLOCK, 0, stream>>>(S, o_tmin, d_tmax, n_ptr, n_fixed, cursor, hit_a, hit_inst, stats, fetch_th, sched, order, n_heavy_ptr, cap, vis_pid, vis, vmask);
         else trace_kernel<false, true><<<grid, TRACE_BLOCK, 0, stream>>>(S, o_tmin, d_tmax, n_ptr, n_fixed, cursor, hit_a, hit_inst, stats, fetch_th, sched, order, n_heavy_ptr, cap, vis_pid, vis, vmask);

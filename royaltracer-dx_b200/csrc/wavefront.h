@@ -50,8 +50,6 @@ struct WaveBuffers {
     // the DI visibility rays of a part are traced on a side stream, beside the part's indirect bounces (they are only read by k_finalize):
     // their persistent CTAs take the SM slots the closest-hit launches leave idle while their last long rays drain
     cudaStream_t aux_sh[WAVE_MAX_PARTS] = {}; cudaEvent_t ev_sh_fork[WAVE_MAX_PARTS] = {}, ev_sh_join[WAVE_MAX_PARTS] = {};
-    bool shadow_overlap = true;
-    int part_rows = -1;                      // concurrent parts own interleaved chunks of this many image rows (< 0: chosen per frame size, 0: contiguous ranges)
     float4* state = nullptr;           // NSTATE * n_paths
     uint2* seeds = nullptr;            // n_paths: RNG state (StateView::seed)
     RayQueue q[2];                     // closest-hit ray queues (ping-pong)

@@ -543,71 +543,91 @@ def test_tlas_refit_matches_rebuild_and_oracle(rtdx, orc):
     ctx.close()
 
 
-def test_concurrent_pass_parts_match_the_oracle(rtdx, orc):
-    """RTX_OPT_PASS_PARTS / RTX_OPT_PART_ROWS: a pass of >= 65536 paths is cut into path ranges (contiguous, or interleaved chunks of image
-    rows) that run on separate CUDA streams; ray counts and the accumulated radiance stay bit-identical to the oracle for 1..4 parts
-    (paths never interact before the accumulation)."""
+def test_interleaved_and_contiguous_pass_parts_match_the_oracle(rtdx, orc):
+    """RTX_OPT_PASS_PARTS: a pass of >= 65536 paths is cut into path ranges (interleaved chunks of image rows when a chunk of <= 32 rows
+    divides the frame evenly among the parts, else contiguous ranges) that run on separate CUDA streams; ray counts and the accumulated
+    radiance stay bit-identical to the oracle for 1..4 parts (paths never interact before the accumulation)."""
     sc = rtdx.scenes.mesh_room(n=16)
-    W, H, bounces = 384, 192, 3                                                            # 73 728 paths
-    ctx, up = _upload(rtdx, sc, W, H, bounces=bounces)
-    osc = orc.OracleScene(sc, up["props"], up["lights"])
-    ref, octr = osc.render(up["camera"], W, H, 0, 1, bounces=bounces, flags=0)
-    for parts, rows in [(1, 0xffffffff), (2, 0xffffffff), (3, 0xffffffff), (4, 0xffffffff), (2, 0), (3, 0), (4, 0), (2, 1), (3, 4), (4, 12), (3, 5)]:
-        ctx.set_option(rtdx.OPT_PASS_PARTS, parts)
-        ctx.set_option(rtdx.OPT_PART_ROWS, rows)       # RTX_OPT_PART_ROWS: interleaved chunks of rows (automatic / contiguous / given / not a divisor)
-        ctx.reset_accum(); ctx.reset_counters()
-        ctx.render_pass(0, 1); ctx.synchronize()
-        cnt = ctx.counters()
-        assert cnt["closest_rays"] == octr["closest_rays"] and cnt["shadow_rays"] == octr["shadow_rays"], (parts, rows, cnt, octr)
-        assert (bits(ctx.read_accum()) != bits(ref)).sum() == 0, (parts, rows)
-    ctx.close()
+    bounces = 3
+    # 384 x 192 = 73 728 paths: every part count interleaves; 384 x 191 = 73 344 paths: 191 is prime, so the parts are contiguous ranges
+    for (W, H), part_counts in (((384, 192), (1, 2, 3, 4)), ((384, 191), (2, 3, 4))):
+        ctx, up = _upload(rtdx, sc, W, H, bounces=bounces)
+        osc = orc.OracleScene(sc, up["props"], up["lights"])
+        ref, octr = osc.render(up["camera"], W, H, 0, 1, bounces=bounces, flags=0)
+        for parts in part_counts:
+            ctx.set_option(rtdx.OPT_PASS_PARTS, parts)
+            ctx.reset_accum(); ctx.reset_counters()
+            ctx.render_pass(0, 1); ctx.synchronize()
+            cnt = ctx.counters()
+            assert cnt["closest_rays"] == octr["closest_rays"] and cnt["shadow_rays"] == octr["shadow_rays"], (W, H, parts, cnt, octr)
+            assert (bits(ctx.read_accum()) != bits(ref)).sum() == 0, (W, H, parts)
+        ctx.close()
     # several samples per pass: the paths of a pass are (sample, pixel) pairs, the chunks are cut in that space
     W2, H2, spp = 192, 96, 4                                                               # 73 728 paths again
     ctx, up = _upload(rtdx, sc, W2, H2, bounces=bounces, samples_per_pass=spp)
     ref2, octr2 = osc.render(up["camera"], W2, H2, 0, spp, bounces=bounces, flags=0)
-    for parts, rows in [(1, 0xffffffff), (2, 0xffffffff), (3, 0xffffffff), (2, 0), (4, 3)]:
-        ctx.set_option(rtdx.OPT_PASS_PARTS, parts); ctx.set_option(rtdx.OPT_PART_ROWS, rows)
+    for parts in (1, 2, 3, 4):
+        ctx.set_option(rtdx.OPT_PASS_PARTS, parts)
         ctx.reset_accum(); ctx.reset_counters()
         ctx.render_pass(0, spp); ctx.synchronize()
         cnt = ctx.counters()
-        assert cnt["closest_rays"] == octr2["closest_rays"] and cnt["shadow_rays"] == octr2["shadow_rays"], (parts, rows, cnt, octr2)
-        assert (bits(ctx.read_accum()) != bits(ref2)).sum() == 0, (parts, rows)
+        assert cnt["closest_rays"] == octr2["closest_rays"] and cnt["shadow_rays"] == octr2["shadow_rays"], (parts, cnt, octr2)
+        assert (bits(ctx.read_accum()) != bits(ref2)).sum() == 0, parts
     ctx.close()
 
 
-def test_graph_replay_and_trace_order_do_not_change_the_image(rtdx, orc):
-    """RTX_OPT_PASS_GRAPH / RTX_OPT_QUEUE_LPT / RTX_OPT_SHADOW_OVERLAP (DI visibility rays on a side stream): the third and later passes of a static configuration replay a captured CUDA graph (the
-    sample index comes from a device word), and the traversal kernels claim rays longest-first through the queue's order array.  Six
-    accumulated samples are bit-identical with both on (default), graph off, order off — and equal to the oracle's six samples; the
-    kernel-launch count is the same whether a pass was launched directly or replayed."""
-    sc = rtdx.scenes.mesh_room(n=16)
+def test_graph_replay_shadow_stream_and_trace_order_do_not_change_the_image(rtdx, orc):
+    """RTX_OPT_PASS_GRAPH: the third and later passes of a static configuration replay a captured CUDA graph (the sample index comes
+    from a device word).  The DI visibility rays of a pass are traced on a side stream, or in sequence when RTX_OPT_TRACE_STATS is on
+    (which also runs without a graph, as one part).  The traversal kernels claim rays longest-first through the queue's order array
+    where the scene's heavy instances separate anything (mesh_room), and in emission order where they do not (cornell: one model, so
+    its heavy box is the scene box).  For each scene six accumulated samples are bit-identical by default, with the graph off and with
+    statistics on — and equal to the oracle's six samples; the kernel-launch count is the same whether a pass was launched directly or
+    replayed."""
     W, H, bounces, n_samples = 384, 192, 3, 6
-    ctx, up = _upload(rtdx, sc, W, H, bounces=bounces)
-    osc = orc.OracleScene(sc, up["props"], up["lights"])
-    ref = None
-    for s in range(n_samples):
-        img, _ = osc.render(up["camera"], W, H, s, 1, bounces=bounces, flags=0)
-        ref = img if ref is None else ref + img               # gPermanentData += sample, in sample order (F20)
-    results = {}
-    for name, opts in (("default", {}), ("no graph", {rtdx.OPT_PASS_GRAPH: 0}), ("emission order", {rtdx.OPT_QUEUE_LPT: 0}),
-                       ("shadow rays in sequence", {rtdx.OPT_SHADOW_OVERLAP: 0}), ("in sequence, no graph", {rtdx.OPT_SHADOW_OVERLAP: 0, rtdx.OPT_PASS_GRAPH: 0})):
-        ctx.set_option(rtdx.OPT_PASS_GRAPH, 1); ctx.set_option(rtdx.OPT_QUEUE_LPT, 1); ctx.set_option(rtdx.OPT_SHADOW_OVERLAP, 1)
-        for k, v in opts.items():
-            ctx.set_option(k, v)
-        ctx.reset_accum(); ctx.reset_counters()
-        per_pass = []
+    for sc in (rtdx.scenes.mesh_room(n=16), rtdx.scenes.cornell()):
+        ctx, up = _upload(rtdx, sc, W, H, bounces=bounces)
+        osc = orc.OracleScene(sc, up["props"], up["lights"])
+        ref = None
         for s in range(n_samples):
-            before = ctx.counters()["kernel_launches"]
-            ctx.render_pass(s, 1)
-            per_pass.append(ctx.counters()["kernel_launches"] - before)
-        ctx.synchronize()
-        results[name] = (ctx.read_accum(), ctx.counters(), per_pass)
-        assert len(set(per_pass)) == 1 and per_pass[0] > 20, (name, per_pass)
-    base = results["default"]
-    assert (bits(base[0]) != bits(ref)).sum() == 0
-    for name, (img, cnt, per_pass) in results.items():
-        assert np.array_equal(bits(img), bits(base[0])), name
-        assert cnt["closest_rays"] == base[1]["closest_rays"] and cnt["shadow_rays"] == base[1]["shadow_rays"], name
+            img, _ = osc.render(up["camera"], W, H, s, 1, bounces=bounces, flags=0)
+            ref = img if ref is None else ref + img               # gPermanentData += sample, in sample order (F20)
+        results = {}
+        # (name, options, path ranges per pass): a pass with statistics runs as one range
+        for name, opts, parts in (("default", {}, 2), ("no graph", {rtdx.OPT_PASS_GRAPH: 0}, 2),
+                                  ("statistics, shadow rays in sequence", {rtdx.OPT_TRACE_STATS: 1}, 1)):
+            ctx.set_option(rtdx.OPT_PASS_GRAPH, 1); ctx.set_option(rtdx.OPT_TRACE_STATS, 0)
+            for k, v in opts.items():
+                ctx.set_option(k, v)
+            ctx.reset_accum(); ctx.reset_counters()
+            per_pass = []
+            for s in range(n_samples):
+                before = ctx.counters()["kernel_launches"]
+                ctx.render_pass(s, 1)
+                per_pass.append(ctx.counters()["kernel_launches"] - before)
+            ctx.synchronize()
+            results[name] = (ctx.read_accum(), ctx.counters(), per_pass)
+            assert len(set(per_pass)) == 1 and per_pass[0] > 10 * parts, (sc.name, name, per_pass)
+        base = results["default"]
+        assert (bits(base[0]) != bits(ref)).sum() == 0, sc.name
+        for name, (img, cnt, per_pass) in results.items():
+            assert np.array_equal(bits(img), bits(base[0])), (sc.name, name)
+            assert cnt["closest_rays"] == base[1]["closest_rays"] and cnt["shadow_rays"] == base[1]["shadow_rays"], (sc.name, name)
+        ctx.close()
+
+
+def test_set_option_rejects_unknown_options_and_part_counts(rtdx):
+    """rtx_set_option fails with RTX_ERR_ARG for an option value no RTX_OPT_* names (among them 5..9, 11 and 12, which named launch
+    tuning options once) and for a RTX_OPT_PASS_PARTS count outside 1..4; the context stays usable."""
+    ctx, _ = _upload(rtdx, rtdx.scenes.cornell(), 64, 64, bounces=2)
+    for option in (5, 6, 7, 8, 9, 11, 12, 0, 15):
+        with pytest.raises(rtdx.RtxError, match="unknown option"):
+            ctx.set_option(option, 1)
+    for parts in (0, 5):
+        with pytest.raises(rtdx.RtxError, match="RTX_OPT_PASS_PARTS"):
+            ctx.set_option(rtdx.OPT_PASS_PARTS, parts)
+    ctx.set_option(rtdx.OPT_PASS_PARTS, 4)
+    ctx.render_pass(0, 1); ctx.synchronize()
     ctx.close()
 
 

@@ -108,16 +108,15 @@ def test_abi_library_exports_every_declared_symbol(rtdx):
         assert hasattr(host, name)
 
 
-def test_python_constants_are_exactly_the_header_flags_and_options(rtdx):
+def test_python_constants_are_exactly_the_header_flags_and_kept_options(rtdx):
     """include/rtx_b200.h defines exactly these RTX_FLAG_* / RTX_OPT_* names, and each has a Python constant of the same value (the
     bindings of tests and bench)."""
     import re
     hdr = open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "include", "rtx_b200.h")).read()
     defs = dict((m.group(1), int(m.group(2), 0)) for m in re.finditer(r"#define\s+RTX_((?:FLAG|OPT)_\w+)\s+(0x[0-9a-fA-F]+|\d+)u", hdr))
     assert sorted(defs) == sorted(["FLAG_JITTER", "FLAG_LAMBERT_ONLY", "FLAG_RESTIR", "FLAG_LEGACY_RR", "FLAG_FAST_MATH"] + [
-        "OPT_TRACE_STATS", "OPT_STAGE_TIMING", "OPT_PASS_PARTS", "OPT_TLAS_REBUILD", "OPT_TRACE_FETCH_TH", "OPT_TRACE_SCHED",
-        "OPT_TRACE_WAVES", "OPT_QUEUE_LPT", "OPT_TRACE_CTAS", "OPT_PASS_GRAPH", "OPT_SHADOW_OVERLAP", "OPT_PART_ROWS",
-        "OPT_PASS_PIPELINE", "OPT_FRAME_PIPELINE"])
+        "OPT_TRACE_STATS", "OPT_STAGE_TIMING", "OPT_PASS_PARTS", "OPT_TLAS_REBUILD", "OPT_PASS_GRAPH", "OPT_PASS_PIPELINE",
+        "OPT_FRAME_PIPELINE"])
     for name, value in defs.items():
         assert getattr(rtdx, name) == value, name
 

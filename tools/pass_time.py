@@ -21,7 +21,7 @@ ap.add_argument("--flags", type=int, default=0)
 ap.add_argument("--spp", type=int, default=1, help="samples per pass (paths in flight = W*H*spp)")
 ap.add_argument("--refit", type=int, default=0, help="call rtx_set_instances this many times after the upload (TLAS refit)")
 ap.add_argument("--tag", default="")
-ap.add_argument("--opt", action="append", default=[], help="engine option NAME=VALUE (rtdx.OPT_<NAME>), e.g. PASS_PARTS=1 TRACE_SCHED=0x060808")
+ap.add_argument("--opt", action="append", default=[], help="engine option NAME=VALUE (rtdx.OPT_<NAME>), e.g. PASS_PARTS=1 PASS_GRAPH=0")
 a = ap.parse_args()
 stream = torch.cuda.Stream(); torch.cuda.set_stream(stream)
 sc = rtdx.scenes.mesh_room(n=a.side) if a.scene == "mesh" else rtdx.scenes.instanced_blobs()

@@ -26,11 +26,10 @@ import os
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import rtdx  # noqa: E402
-lpt = int(sys.argv[1]) if len(sys.argv) > 1 else 1
 sc = rtdx.scenes.mesh_room(n=296)
 ctx = rtdx.Context(1920, 1080, bounces=6)
 ctx.upload_scene(sc)
-ctx.set_option(rtdx.OPT_PASS_PARTS, 1); ctx.set_option(rtdx.OPT_QUEUE_LPT, lpt)
+ctx.set_option(rtdx.OPT_PASS_PARTS, 1)
 ctx.render_pass(0, 1); ctx.synchronize()
-print("=== pass lpt=%d" % lpt, flush=True)
+print("=== pass", flush=True)
 ctx.render_pass(1, 1); ctx.synchronize()

@@ -17,7 +17,7 @@ ap.add_argument("--bounces", type=int, default=6)
 ap.add_argument("--passes", type=int, default=8)
 ap.add_argument("--flags", type=int, default=0)
 ap.add_argument("--tag", default="")
-ap.add_argument("--opt", action="append", default=[], help="engine option NAME=VALUE (rtdx.OPT_<NAME>), e.g. PASS_PARTS=1 TRACE_SCHED=0x060808")
+ap.add_argument("--opt", action="append", default=[], help="engine option NAME=VALUE (rtdx.OPT_<NAME>), e.g. PASS_PARTS=1 PASS_GRAPH=0")
 a = ap.parse_args()
 sc = rtdx.scenes.mesh_room(n=a.side) if a.scene == "mesh" else (rtdx.scenes.instanced_blobs() if a.scene == "inst" else rtdx.scenes.cornell())
 ctx = rtdx.Context(a.width, a.height, bounces=a.bounces, flags=a.flags)
