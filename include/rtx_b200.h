@@ -106,7 +106,8 @@ rtx_status rtx_blas_info_get(rtx_ctx*, uint32_t model_id, rtx_blas_info* out);
  * the brute-force definition in both modes.
  * Stream order: like every entry point, ordered after all passes already queued (pipelined ones included); work queued after the call
  * sees the new geometry, captured pass graphs included (no recapture).  The call does not reset the accumulation (only a view change
- * does) and does not touch the emissive-triangle list: a caller that deforms an emissive model collects and sets it again.
+ * does) and does not touch the emissive-triangle list: a caller that deforms an emissive model refreshes it on the device with
+ * rtx_collect_emissive_triangles (or collects it on the host and sets it again).
  * Errors: RTX_ERR_ARG before any device work for a null context, an unknown model, a vertex count that differs from the upload, an
  * unknown mode, a null pointer with a nonzero count, and (_device) memory that is not device or managed memory of cfg.device.
  * RTX_UPDATE_REBUILD re-runs the traversal-stack depth check of rtx_set_instances and returns RTX_ERR_STATE as it does. */
@@ -128,6 +129,26 @@ rtx_status rtx_set_materials(rtx_ctx*, const rtx_material* m, uint32_t n);
 rtx_status rtx_set_instances(rtx_ctx*, const rtx_instance_desc* descs, const rtx_instance_props* props, uint32_t n);
 /* binding t6 (rdn/Renderer.cpp:2237-2280) */
 rtx_status rtx_set_emissive_triangles(rtx_ctx*, const rtx_light_triangle* l, uint32_t n);
+/* Binding t6 built on the device (CollectEmissiveTriangles + CreateEmissiveTrianglesBuffer, rdn/Renderer.cpp:2123-2243) from the
+ * context's current state: every model's vertices as they are now (after any rtx_update_model*), the material ids, the materials and
+ * the instance list of the last rtx_set_instances.  Written into the same light buffer rtx_set_emissive_triangles fills: whichever of
+ * the two calls ran last defines t6.  For finite positions and in-range material ids the records, their order and their count equal
+ * the host collection byte for byte: instances in list order and their model's triangles in index order, a triangle kept when its
+ * three face-vertex material ids are equal and that material's Ke0+Ke1+Ke2 > 0; the weight area * (Ke sum / 3) in the reference's
+ * operation order; a stable sort by descending weight; the sequential binary32 sums of the weights and of weight / total; the last
+ * cdf set to 1.  A slot past the material ids reads id 0 and an id past the materials reads a zero material, as in the shading
+ * kernels.  No emitter: count 0 and one zero record, as rtx_set_emissive_triangles(ctx, NULL, 0).  n_out (may be NULL) receives the
+ * record count, known on the host.
+ * Stream order: like every entry point, after all passes already queued (pipelined ones included); work queued after the call sees the
+ * new list.  Only the first call after rtx_set_material_ids, rtx_set_materials or rtx_upload_model (it rebuilds the per-model index of
+ * emissive triangles) and a call whose record or instance count exceeds every earlier call's synchronise the host or allocate; the
+ * per-frame call after rtx_update_model* or an rtx_set_instances of the same models does neither.
+ * Errors: RTX_ERR_ARG for a null context; RTX_ERR_STATE, with no device work done, when materials or material ids were never set or
+ * no instance list is current (never set, or invalidated by rtx_upload_model). */
+rtx_status rtx_collect_emissive_triangles(rtx_ctx*, uint32_t* n_out);
+/* Reads t6 back, whichever call set it: *n_out (may be NULL) = the record count; with out non-NULL and cap >= n the n records are
+ * copied and the call synchronises like rtx_read_accum.  cap < n with out non-NULL: RTX_ERR_ARG. */
+rtx_status rtx_read_emissive_triangles(rtx_ctx*, rtx_light_triangle* out, uint32_t cap, uint32_t* n_out);
 /* binding b0 (rdn/Renderer.cpp:1722-1768); a view change resets the accumulation (Pass_spat_di_v7.hlsl:407-423) */
 rtx_status rtx_set_camera(rtx_ctx*, const rtx_camera_params*);
 /* replaces the DispatchRays sequence (rdn/Renderer.cpp:611-673): renders samples [first_sample, first_sample+n_samples)

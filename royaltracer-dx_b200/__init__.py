@@ -60,7 +60,8 @@ class RtxBlasInfo(C.Structure):
 # every symbol include/rtx_b200.h declares (tests check the library exports all of them)
 ABI_SYMBOLS = ["rtx_last_error", "rtx_create", "rtx_destroy", "rtx_upload_model", "rtx_update_model", "rtx_update_model_device",
                "rtx_blas_info_get", "rtx_set_material_ids",
-               "rtx_set_materials", "rtx_set_instances", "rtx_set_emissive_triangles", "rtx_set_camera", "rtx_render_pass",
+               "rtx_set_materials", "rtx_set_instances", "rtx_set_emissive_triangles", "rtx_collect_emissive_triangles",
+               "rtx_read_emissive_triangles", "rtx_set_camera", "rtx_render_pass",
                "rtx_reset_accum", "rtx_synchronize", "rtx_read_accum", "rtx_read_output", "rtx_read_output_async", "rtx_wait_output", "rtx_set_resolve_source",
                "rtx_accum_device_ptr", "rtx_trace",
                "rtx_trace_device", "rtx_trace_stats", "rtx_get_counters", "rtx_reset_counters", "rtx_last_pass_ms", "rtx_last_pass_stage_ms", "rtx_set_option", "rtx_debug_pixel",
@@ -98,6 +99,8 @@ def load_library():
     lib.rtx_set_materials.argtypes = [vp, vp, u32]
     lib.rtx_set_instances.argtypes = [vp, vp, vp, u32]
     lib.rtx_set_emissive_triangles.argtypes = [vp, vp, u32]
+    lib.rtx_collect_emissive_triangles.argtypes = [vp, C.POINTER(u32)]
+    lib.rtx_read_emissive_triangles.argtypes = [vp, vp, u32, C.POINTER(u32)]
     lib.rtx_set_camera.argtypes = [vp, vp]
     lib.rtx_render_pass.argtypes = [vp, u32, u32]
     lib.rtx_reset_accum.argtypes = [vp]
@@ -302,6 +305,22 @@ class Context:
     def set_emissive_triangles(self, lights):
         a = np.ascontiguousarray(lights, dtype=light_dt)
         self._check(self.lib.rtx_set_emissive_triangles(self.handle, _ptr(a), a.size))
+
+    def collect_emissive_triangles(self):
+        """Builds the light list on the device from the models' current vertices, the materials and the last instance list (the bytes
+        of collect_emissive_triangles(scene) over the same state) and makes it the one passes sample; returns the record count."""
+        n = C.c_uint32()
+        self._check(self.lib.rtx_collect_emissive_triangles(self.handle, C.byref(n)))
+        return n.value
+
+    def read_emissive_triangles(self):
+        """The light list passes sample (set or collected), as a light_dt array."""
+        n = C.c_uint32()
+        self._check(self.lib.rtx_read_emissive_triangles(self.handle, None, 0, C.byref(n)))
+        out = np.zeros(n.value, dtype=light_dt)
+        if n.value:
+            self._check(self.lib.rtx_read_emissive_triangles(self.handle, _ptr(out), out.size, C.byref(n)))
+        return out
 
     def set_camera(self, cam):
         a = np.ascontiguousarray(cam, dtype=camera_dt)

@@ -9,6 +9,7 @@
 #include "restir.h"
 #include <stdlib.h>
 
+#include "lights.h"
 #include "trace.h"
 #include "wavefront.h"
 
@@ -53,6 +54,8 @@ struct rtx_ctx {
     cudaStream_t copy_stream = nullptr; cudaEvent_t ev_resolved = nullptr, ev_copied = nullptr; bool copy_pending = false;
     BlasRef* d_blas = nullptr; BlasBounds* d_bounds = nullptr; ModelRef* d_model_refs = nullptr; uint32_t n_tables = 0;
     rtx_light_triangle* d_lights = nullptr; uint32_t n_lights = 0;
+    // rtx_collect_emissive_triangles: the emissive index is rebuilt after rtx_set_material_ids / rtx_set_materials / rtx_upload_model
+    LightBuffers lb; bool light_index_stale = true;
     rtx_camera_params cam; bool have_cam = false;
     WaveBuffers wb; bool wb_ready = false;
     RestirBuffers rs; bool rs_ready = false;
@@ -195,6 +198,7 @@ extern "C" void rtx_destroy(rtx_ctx* c) {
     if (c->h_overflow) cudaFreeHost(c->h_overflow);
     for (auto& f : c->fs) free_frame_set(f);
     free_tables(c);
+    lights_free(c->lb);
     if (c->copy_stream) { cudaStreamSynchronize(c->copy_stream); cudaStreamDestroy(c->copy_stream); }
     if (c->ev_resolved) cudaEventDestroy(c->ev_resolved);
     if (c->ev_copied) cudaEventDestroy(c->ev_copied);
@@ -259,6 +263,7 @@ extern "C" rtx_status rtx_upload_model(rtx_ctx* c, const rtx_vertex* v, uint32_t
     RTX_CK(cudaGetLastError());
     c->launches += 9;
     c->models.push_back(m);
+    c->light_index_stale = true;
     // the per-model tables are rebuilt by the next rtx_set_instances; until then there is no valid TLAS (rendering or tracing in
     // between returns RTX_ERR_STATE instead of handing freed tables to the kernels)
     free_tables(c);
@@ -297,6 +302,7 @@ extern "C" rtx_status rtx_set_material_ids(rtx_ctx* c, const uint32_t* ids, uint
     if (!c || (!ids && n)) return fail(RTX_ERR_ARG, "rtx_set_material_ids: null argument");
     RTX_ENTER(c);
     c->n_material_ids = n;
+    c->light_index_stale = true;
     return upload(&c->d_material_ids, ids, n, c->stream, &c->cap_material_ids);
 }
 
@@ -304,6 +310,7 @@ extern "C" rtx_status rtx_set_materials(rtx_ctx* c, const rtx_material* m, uint3
     if (!c || (!m && n)) return fail(RTX_ERR_ARG, "rtx_set_materials: null argument");
     RTX_ENTER(c);
     c->n_materials = n;
+    c->light_index_stale = true;
     return upload(&c->d_materials, m, n, c->stream, &c->cap_materials);
 }
 
@@ -683,6 +690,50 @@ static SceneAS make_as(rtx_ctx* c, int set = 0) {
     a.overflow = c->d_overflow;
     a.num_sms = c->num_sms;
     return a;
+}
+
+// Binding t6 from the scene as it is now (csrc/lights.cu).  Only a stale emissive index (material ids, materials or models changed)
+// and a record count or instance count above every earlier call's make the call synchronise or allocate.
+extern "C" rtx_status rtx_collect_emissive_triangles(rtx_ctx* c, uint32_t* n_out) {
+    if (!c) return fail(RTX_ERR_ARG, "rtx_collect_emissive_triangles: null context");
+    if (!c->n_instances || !c->fs[0].tlas.nodes) return fail(RTX_ERR_STATE, "rtx_collect_emissive_triangles: no instances");
+    if (!c->d_materials || !c->d_material_ids) return fail(RTX_ERR_STATE, "rtx_collect_emissive_triangles: materials not set");
+    RTX_ENTER(c);
+    const SceneData S = scene_data(c);
+    if (c->light_index_stale) {
+        std::vector<ModelRef> mr(c->models.size());
+        for (size_t i = 0; i < mr.size(); i++) {
+            memset(&mr[i], 0, sizeof mr[i]);
+            mr[i].mat_offset = c->models[i].mat_offset; mr[i].n_tris = c->models[i].n_tris;
+        }
+        RTX_CK(lights_build_index(c->lb, mr, S, c->stream, &c->launches));
+        c->light_index_stale = false;
+    }
+    uint64_t n = 0;
+    for (uint32_t m : c->tlas_models) n += c->lb.count[m];
+    if (n > 0xFFFFFFFFull) return fail(RTX_ERR_STATE, "rtx_collect_emissive_triangles: more than 2^32 - 1 emissive triangles");
+    if (!c->d_lights || c->cap_lights < (n ? n : 1)) {     // (passes queued before may still read the old list)
+        if (c->d_lights) { RTX_CK(cudaStreamSynchronize(c->stream)); cudaFree(c->d_lights); c->d_lights = nullptr; c->cap_lights = 0; }
+        RTX_CK(cudaMalloc((void**)&c->d_lights, (n ? n : 1) * sizeof(rtx_light_triangle)));
+        c->cap_lights = n ? n : 1;
+    }
+    if (n == 0) RTX_CK(cudaMemsetAsync(c->d_lights, 0, sizeof(rtx_light_triangle), c->stream));     // as rtx_set_emissive_triangles(NULL, 0)
+    else RTX_CK(lights_collect(c->lb, S, c->n_instances, (uint32_t)n, c->d_lights, c->stream, &c->launches));
+    c->n_lights = (uint32_t)n;
+    if (n_out) *n_out = (uint32_t)n;
+    return RTX_OK;
+}
+
+extern "C" rtx_status rtx_read_emissive_triangles(rtx_ctx* c, rtx_light_triangle* out, uint32_t cap, uint32_t* n_out) {
+    if (!c) return fail(RTX_ERR_ARG, "rtx_read_emissive_triangles: null context");
+    const uint32_t n = c->n_lights;
+    if (n_out) *n_out = n;
+    if (!out || n == 0) return RTX_OK;
+    if (cap < n) return fail(RTX_ERR_ARG, "rtx_read_emissive_triangles: cap is less than the record count");
+    RTX_ENTER(c);
+    RTX_CK(cudaMemcpyAsync(out, c->d_lights, (size_t)n * sizeof(rtx_light_triangle), cudaMemcpyDeviceToHost, c->stream));
+    RTX_CK(cudaStreamSynchronize(c->stream));
+    return RTX_OK;
 }
 
 // Reads the context's overflow word behind everything queued on the stream; a raised word fails the call ONCE and is cleared, so that
