@@ -57,7 +57,10 @@ struct rtx_ctx {
     // rtx_collect_emissive_triangles: the emissive index is rebuilt after rtx_set_material_ids / rtx_set_materials / rtx_upload_model
     LightBuffers lb; bool light_index_stale = true;
     rtx_camera_params cam; bool have_cam = false;
-    WaveBuffers wb; bool wb_ready = false;
+    int cam_version = 0;                    // counts rtx_set_camera calls (Lane::cam_version)
+    // gPermanentData, gOutput (RGBA8) and what the resolve reads: allocated with lane 0's buffers, shared by both lanes
+    float4* d_accum = nullptr; uint8_t* d_output = nullptr;
+    const float4* resolve_source = nullptr; // rtx_set_resolve_source: an external accumulation buffer (the multi-GPU sum) to resolve instead
     RestirBuffers rs; bool rs_ready = false;
     float4* d_trace_o = nullptr; float4* d_trace_d = nullptr; float4* d_trace_ha = nullptr; uint32_t* d_trace_hi = nullptr;
     rtx_hit* d_trace_out = nullptr; uint32_t trace_cap = 0;
@@ -73,33 +76,40 @@ struct rtx_ctx {
     void* comm = nullptr; int comm_rank = 0, comm_world = 1;
     float4* d_total = nullptr;              // root only: the sum over ranks; rtx_read_output* resolve it
     cudaEvent_t ev_pass = nullptr, ev_reduced = nullptr;
+    bool reduce_pending = false;            // the last rtx_reduce_accum may still read gPermanentData: the next accumulation waits for ev_reduced
     float heavy_lo[3] = {0, 0, 0}, heavy_hi[3] = {0, 0, 0}; bool heavy_valid = false;   // SceneData::heavy_* (queue order only)
     uint64_t launches = 0;
-    PassTiming timing;
     bool trace_stats = false;
     bool pass_timed = false;
     // Pipelined passes (RTX_OPT_PASS_PIPELINE): rtx_render_pass calls that follow each other with no other call in between alternate
-    // between two sets of pass buffers ("lanes": wb and wb2) on two private streams, each pass as ONE path range, so that the start and
-    // the tail of a pass overlap the middle of the other one.  gPermanentData is shared: the k_accumulate launches are chained through
-    // ev_acc in call order, so the sums are bit-identical to passes run one after the other.  The API stays stream-ordered: a lane
-    // starts behind ev_state (whatever other entry points queued on the caller's stream), and the caller's stream is made to wait for
-    // every pass's accumulation (no host wait).  The first pass after any other call runs as before (B.parts path ranges on the
-    // caller's stream).
+    // between two lanes (lane[0] and lane[1]: a set of pass buffers and a private stream each), each pass as ONE path range, so that
+    // the start and the tail of a pass overlap the middle of the other one.  gPermanentData is shared: the k_accumulate launches are
+    // chained through the lanes' ev_acc in call order, so the sums are bit-identical to passes run one after the other.  The API stays
+    // stream-ordered: a lane starts behind ev_state (whatever other entry points queued on the caller's stream), and the caller's
+    // stream is made to wait for every pass's accumulation (no host wait).  The first pass after any other call runs as before
+    // (B.parts path ranges on the caller's stream, in lane 0's buffers).
     // Pipelined FRAMES (RTX_OPT_FRAME_PIPELINE): a per-frame loop in the reference's order — rtx_set_instances, rtx_set_camera,
     // rtx_render_pass, rtx_read_output_async — with a TLAS that fits one node (<= 8 instances: BASELINE config C2) keeps two sets of the
-    // per-frame state (fs[0] and fs[1], and the camera blocks), one per lane: the calls of frame k+1 write the set of the lane frame k-1
-    // used and queue on that lane's stream, so frame k+1 starts under the tail of frame k.  Every other call pattern takes the plain
-    // path above (enter() first copies fs[1] back into fs[0] if it is the newer one).
+    // per-frame state (fs[0] and fs[1], and the lanes' camera blocks), one per lane: the calls of frame k+1 write the set of the lane
+    // frame k-1 used and queue on that lane's stream, so frame k+1 starts under the tail of frame k.  Every other call pattern takes
+    // the plain path above (enter() first copies fs[1] back into fs[0] if it is the newer one).
     bool frame_pipeline = true, frame_seq_ok = false, resolve_pending = false;
     cudaEvent_t ev_fset = nullptr; bool fset_pending = false;       // behind the last fast rtx_set_instances / rtx_set_camera on a lane stream
     int pending_lane = -1;              // >= 0: the fast rtx_set_instances of this frame prepared that lane
     int cur_set = 0;                    // which set of per-frame instance state (fs) is the newest
-    int lane_read_set[2] = {0, 0};      // the set the last pass of each lane read
-    int cam_version = 0, cam_block_version[2] = {0, 0};   // the camera blocks of the two lanes (wb.cam, wb2.cam) against the latest rtx_set_camera
-    WaveBuffers wb2; bool wb2_ready = false, wb2_refused = false;
-    cudaStream_t lane_stream[2] = {nullptr, nullptr}; cudaEvent_t ev_acc[2] = {nullptr, nullptr}, ev_state = nullptr;
-    PassTiming timing2;
-    bool pipeline = true, in_sequence = false, main_dirty = true, reduce_pending = false;
+    // Lane 0's buffers also serve every pass that is not pipelined, the ReSTIR frame and rtx_trace; they are allocated on first use.
+    // Lane 1's are allocated when a pipelined pass first needs them, and only if they take less than a quarter of the free memory.
+    struct Lane {
+        WaveBuffers wb; bool ready = false;
+        cudaStream_t stream = nullptr;
+        cudaEvent_t ev_acc = nullptr;   // behind the lane's last accumulation
+        PassTiming timing;              // lane 0: RTX_OPT_STAGE_TIMING / TRACE_STATS and every event; lane 1: only ev[0], ev[1]
+        int read_set = 0;               // the set of per-frame instance state (fs) its last pass read
+        int cam_version = 0;            // the rtx_set_camera its camera block (wb.cam) holds
+    } lane[2];
+    bool lane1_refused = false;         // lane 1's buffers could not be allocated: passes are not pipelined
+    cudaEvent_t ev_state = nullptr;
+    bool pipeline = true, in_sequence = false, main_dirty = true;
     int last_lane = 0;
 };
 
@@ -124,12 +134,14 @@ extern "C" rtx_status rtx_comm_destroy(rtx_ctx* c);
 static rtx_status create_resources(rtx_ctx* c) {
     if (c->cfg.stream) c->stream = (cudaStream_t)c->cfg.stream;
     else { RTX_CK(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking)); c->own_stream = true; }
-    for (int i = 0; i < WAVE_MAX_EVENTS; i++) RTX_CK(cudaEventCreate(&c->timing.ev[i]));
-    for (int i = 0; i < 2; i++) RTX_CK(cudaEventCreate(&c->timing2.ev[i]));
-    for (int i = 0; i < 2; i++) RTX_CK(cudaEventCreateWithFlags(&c->ev_acc[i], cudaEventDisableTiming));
+    for (int i = 0; i < 2; i++) {
+        rtx_ctx::Lane& l = c->lane[i];
+        for (int k = 0; k < (i ? 2 : WAVE_MAX_EVENTS); k++) RTX_CK(cudaEventCreate(&l.timing.ev[k]));
+        RTX_CK(cudaEventCreateWithFlags(&l.ev_acc, cudaEventDisableTiming));
+        RTX_CK(cudaStreamCreateWithFlags(&l.stream, cudaStreamNonBlocking));
+    }
     RTX_CK(cudaEventCreateWithFlags(&c->ev_state, cudaEventDisableTiming));
     RTX_CK(cudaEventCreateWithFlags(&c->ev_fset, cudaEventDisableTiming));
-    for (int i = 0; i < 2; i++) RTX_CK(cudaStreamCreateWithFlags(&c->lane_stream[i], cudaStreamNonBlocking));
     RTX_CK(cudaMalloc((void**)&c->d_stats, sizeof(TraceStats)));
     RTX_CK(cudaMemset(c->d_stats, 0, sizeof(TraceStats)));
     RTX_CK(cudaMalloc((void**)&c->d_overflow, sizeof(unsigned int)));
@@ -185,7 +197,7 @@ static void free_frame_set(rtx_ctx::FrameSet& f) {
 extern "C" void rtx_destroy(rtx_ctx* c) {
     if (!c) return;
     cudaSetDevice(c->cfg.device);
-    for (int i = 0; i < 2; i++) if (c->lane_stream[i]) cudaStreamSynchronize(c->lane_stream[i]);
+    for (auto& l : c->lane) if (l.stream) cudaStreamSynchronize(l.stream);
     if (c->stream) cudaStreamSynchronize(c->stream);
     rtx_comm_destroy(c);
     for (auto& m : c->models) {
@@ -193,7 +205,7 @@ extern "C" void rtx_destroy(rtx_ctx* c) {
         if (m.h_bounds) cudaFreeHost(m.h_bounds);
     }
     void* ptrs[] = {c->d_material_ids, c->d_materials, c->d_lights, c->d_trace_o, c->d_trace_d, c->d_trace_ha, c->d_trace_hi,
-                    c->d_trace_out, c->d_stats, c->d_overflow, c->d_trace_rays, c->d_trace_hits, c->d_refit};
+                    c->d_trace_out, c->d_stats, c->d_overflow, c->d_trace_rays, c->d_trace_hits, c->d_refit, c->d_accum, c->d_output};
     for (void* p : ptrs) if (p) cudaFree(p);
     if (c->h_overflow) cudaFreeHost(c->h_overflow);
     for (auto& f : c->fs) free_frame_set(f);
@@ -203,15 +215,16 @@ extern "C" void rtx_destroy(rtx_ctx* c) {
     if (c->ev_resolved) cudaEventDestroy(c->ev_resolved);
     if (c->ev_copied) cudaEventDestroy(c->ev_copied);
     for (auto& sg : c->stage) { if (sg.p) cudaFreeHost(sg.p); if (sg.ev) cudaEventDestroy(sg.ev); }
-    if (c->wb2_ready) wave_free_lane(&c->wb2);
-    if (c->wb_ready) wave_free(&c->wb);
     if (c->rs_ready) restir_free(&c->rs);
-    for (int i = 0; i < WAVE_MAX_EVENTS; i++) if (c->timing.ev[i]) cudaEventDestroy(c->timing.ev[i]);
-    for (int i = 0; i < 2; i++) { if (c->timing2.ev[i]) cudaEventDestroy(c->timing2.ev[i]); if (c->ev_acc[i]) cudaEventDestroy(c->ev_acc[i]); }
+    for (auto& l : c->lane) {
+        if (l.ready) wave_free(&l.wb);
+        for (cudaEvent_t e : l.timing.ev) if (e) cudaEventDestroy(e);
+        if (l.ev_acc) cudaEventDestroy(l.ev_acc);
+        if (l.stream) cudaStreamDestroy(l.stream);
+    }
     if (c->ev_state) cudaEventDestroy(c->ev_state);
     if (c->ev_fset) cudaEventDestroy(c->ev_fset);
     if (c->ev_bounds) cudaEventDestroy(c->ev_bounds);
-    for (int i = 0; i < 2; i++) if (c->lane_stream[i]) cudaStreamDestroy(c->lane_stream[i]);
     if (c->own_stream && c->stream) cudaStreamDestroy(c->stream);
     delete c;
 }
@@ -432,8 +445,8 @@ static rtx_status sync_frame_state(rtx_ctx* c) {
 }
 // is the call part of a per-frame loop that can be pipelined?  (the previous frame ended with rtx_render_pass [+ read-back] and nothing else)
 static bool frame_fast_ok(rtx_ctx* c) {
-    return c->pipeline && c->frame_pipeline && c->frame_seq_ok && c->wb_ready &&
-           !(c->cfg.flags & (RTX_FLAG_LEGACY_RR | RTX_FLAG_RESTIR)) && !c->timing.stage_timing && !c->trace_stats &&
+    return c->pipeline && c->frame_pipeline && c->frame_seq_ok && c->lane[0].ready &&
+           !(c->cfg.flags & (RTX_FLAG_LEGACY_RR | RTX_FLAG_RESTIR)) && !c->lane[0].timing.stage_timing && !c->trace_stats &&
            (uint64_t)c->cfg.width * c->cfg.height * c->cfg.samples_per_pass >= 65536u && lane_buffers(c) && ensure_frame_set(c);
 }
 
@@ -510,11 +523,12 @@ extern "C" rtx_status rtx_set_instances(rtx_ctx* c, const rtx_instance_desc* des
         // the per-frame path of a pipelined frame loop: the state set of the lane this frame will render on, on that lane's stream
         const int L = 1 - c->last_lane;
         rtx_ctx::FrameSet& f = c->fs[L];
-        const cudaStream_t s_ = c->lane_stream[L];
+        const rtx_ctx::Lane &l = c->lane[L], &other = c->lane[1 - L];
+        const cudaStream_t s_ = l.stream;
         if (c->main_dirty) { RTX_CK(cudaEventRecord(c->ev_state, c->stream)); c->main_dirty = false; }
         RTX_CK(cudaStreamWaitEvent(s_, c->ev_state, 0));
-        RTX_CK(cudaStreamWaitEvent(s_, c->ev_acc[L], 0));                                        // the last pass of this lane ...
-        if (c->lane_read_set[1 - L] == L) RTX_CK(cudaStreamWaitEvent(s_, c->ev_acc[1 - L], 0));   // ... and of the other one if it read this set
+        RTX_CK(cudaStreamWaitEvent(s_, l.ev_acc, 0));                                        // the last pass of this lane ...
+        if (other.read_set == L) RTX_CK(cudaStreamWaitEvent(s_, other.ev_acc, 0));           // ... and of the other one if it read this set
         if (L) { Bvh8 t = f0.tlas; t.nodes = f.tlas.nodes; t.prims = f.tlas.prims; f.tlas = t; }  // set 0's counts, levels, bounds
         if ((st = stage_instances(c, descs, props, n, f.d_descs, f.d_props, f.d_inst_model, s_)) != RTX_OK) return st;
         if ((st = update_instance_state(c, f, n, same_models, s_)) != RTX_OK) return st;
@@ -622,10 +636,26 @@ extern "C" rtx_status rtx_set_emissive_triangles(rtx_ctx* c, const rtx_light_tri
     return upload(&c->d_lights, l, n, c->stream, &c->cap_lights);
 }
 
+// lane 0's pass buffers, and with them gPermanentData and gOutput
 static rtx_status ensure_wave(rtx_ctx* c) {
-    if (c->wb_ready) return RTX_OK;
-    RTX_CK(wave_alloc(&c->wb, c->cfg.width, c->cfg.height, c->cfg.samples_per_pass));
-    c->wb_ready = true;
+    rtx_ctx::Lane& l = c->lane[0];
+    if (l.ready) return RTX_OK;
+    const size_t npx = (size_t)c->cfg.width * c->cfg.height;
+    if (!c->d_accum) {
+        RTX_CK(cudaMalloc((void**)&c->d_accum, npx * 16));
+        RTX_CK(cudaMemset(c->d_accum, 0, npx * 16));
+    }
+    if (!c->d_output) RTX_CK(cudaMalloc((void**)&c->d_output, npx * 4));
+    RTX_CK(wave_alloc(&l.wb, c->d_accum, c->cfg.width, c->cfg.height, c->cfg.samples_per_pass));
+    l.ready = true;
+    return RTX_OK;
+}
+
+// the camera of the last rtx_set_camera into the lane's camera block (on stream s), unless the block holds it already
+static rtx_status lane_camera(rtx_ctx* c, rtx_ctx::Lane& l, cudaStream_t s) {
+    if (l.cam_version == c->cam_version) return RTX_OK;
+    RTX_CK(cudaMemcpyAsync(l.wb.cam, &c->cam, sizeof c->cam, cudaMemcpyHostToDevice, s));
+    l.cam_version = c->cam_version;
     return RTX_OK;
 }
 
@@ -649,20 +679,18 @@ extern "C" rtx_status rtx_set_camera(rtx_ctx* c, const rtx_camera_params* cam) {
     c->cam = *cam; c->have_cam = true;
     c->cam_version++;
     if (fast_lane >= 0) {
-        const cudaStream_t s_ = c->lane_stream[fast_lane];      // (already behind ev_state and the lane's last pass: rtx_set_instances)
-        RTX_CK(cudaMemcpyAsync(fast_lane ? c->wb2.cam : c->wb.cam, &c->cam, sizeof c->cam, cudaMemcpyHostToDevice, s_));
-        c->cam_block_version[fast_lane] = c->cam_version;
+        const cudaStream_t s_ = c->lane[fast_lane].stream;      // (already behind ev_state and the lane's last pass: rtx_set_instances)
+        if ((st = lane_camera(c, c->lane[fast_lane], s_)) != RTX_OK) return st;
         if (different) {        // the reset lands between the previous frame's accumulation (and resolve) and this frame's
-            RTX_CK(cudaStreamWaitEvent(s_, c->ev_acc[1 - fast_lane], 0));
+            RTX_CK(cudaStreamWaitEvent(s_, c->lane[1 - fast_lane].ev_acc, 0));
             if (c->resolve_pending) RTX_CK(cudaStreamWaitEvent(s_, c->ev_resolved, 0));
-            RTX_CK(cudaMemsetAsync(c->wb.accum, 0, (size_t)c->cfg.width * c->cfg.height * 16, s_));
+            RTX_CK(cudaMemsetAsync(c->d_accum, 0, (size_t)c->cfg.width * c->cfg.height * 16, s_));
         }
         RTX_CK(cudaEventRecord(c->ev_fset, s_)); c->fset_pending = true;
         return RTX_OK;
     }
-    RTX_CK(cudaMemcpyAsync(c->wb.cam, &c->cam, sizeof c->cam, cudaMemcpyHostToDevice, c->stream));
-    c->cam_block_version[0] = c->cam_version;       // (lane 1's block is brought up to date when a pass runs there)
-    if (different) RTX_CK(cudaMemsetAsync(c->wb.accum, 0, (size_t)c->cfg.width * c->cfg.height * 16, c->stream));
+    if ((st = lane_camera(c, c->lane[0], c->stream)) != RTX_OK) return st;     // (lane 1's block is brought up to date when a pass runs there)
+    if (different) RTX_CK(cudaMemsetAsync(c->d_accum, 0, (size_t)c->cfg.width * c->cfg.height * 16, c->stream));
     return RTX_OK;      // the 512-B copy from pageable memory is staged by the driver before the call returns
 }
 
@@ -750,21 +778,33 @@ static rtx_status check_overflow(rtx_ctx* c) {
     return RTX_OK;
 }
 
-// the second set of pass buffers, allocated when first needed and only if it takes less than a quarter of the free device memory
+// lane 1's pass buffers, allocated when first needed and only if they take less than a quarter of the free device memory
 static bool lane_buffers(rtx_ctx* c) {
-    if (c->wb2_ready) return true;
-    if (c->wb2_refused || !c->wb_ready) return false;
+    rtx_ctx::Lane& l = c->lane[1];
+    if (l.ready) return true;
+    if (c->lane1_refused || !c->lane[0].ready) return false;
     size_t free_b = 0, total_b = 0;
-    const size_t need = (size_t)c->wb.n_paths * 480u;
-    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess || need > free_b / 4) { c->wb2_refused = true; return false; }
-    c->wb2 = WaveBuffers();
-    if (wave_alloc_lane(&c->wb2, c->wb, c->cfg.width, c->cfg.height, c->cfg.samples_per_pass) != cudaSuccess) {
+    const size_t need = (size_t)c->lane[0].wb.n_paths * 480u;
+    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess || need > free_b / 4) { c->lane1_refused = true; return false; }
+    l.wb = WaveBuffers();
+    if (wave_alloc(&l.wb, c->d_accum, c->cfg.width, c->cfg.height, c->cfg.samples_per_pass) != cudaSuccess) {
         cudaGetLastError();
-        wave_free_lane(&c->wb2); c->wb2_refused = true;
+        wave_free(&l.wb); c->lane1_refused = true;
         return false;
     }
-    c->wb2_ready = true;
+    l.ready = true;
     return true;
+}
+
+// One pass of the context's estimator and arithmetic on a lane's buffers, reading set `set` of the per-frame instance state.
+// pipelined: one path range, without the accumulation (the caller chains it behind the other lane's); never the legacy estimator.
+static cudaError_t run_pass(rtx_ctx* c, rtx_ctx::Lane& l, int set, uint32_t first_sample, uint32_t spp, cudaStream_t s, bool pipelined) {
+    const SceneData S = scene_data(c, set);
+    const SceneAS AS = make_as(c, set);
+    if (c->cfg.flags & RTX_FLAG_LEGACY_RR) return wave_render_pass_legacy(l.wb, S, AS, first_sample, spp, s, &c->launches, &l.timing);
+    const auto pass = (c->cfg.flags & RTX_FLAG_FAST_MATH) ? fast::wave_render_pass : wave_render_pass;
+    return pass(l.wb, S, AS, first_sample, spp, s, &c->launches, &l.timing, c->reduce_pending ? c->ev_reduced : nullptr, true,
+                pipelined ? 1 : 0, pipelined);
 }
 
 extern "C" rtx_status rtx_render_pass(rtx_ctx* c, uint32_t first_sample, uint32_t n_samples) {
@@ -777,13 +817,14 @@ extern "C" rtx_status rtx_render_pass(rtx_ctx* c, uint32_t first_sample, uint32_
     if (!c->d_lights && (st = rtx_set_emissive_triangles(c, nullptr, 0)) != RTX_OK) return st;
     if ((st = ensure_wave(c)) != RTX_OK) return st;
     const uint32_t npx = c->cfg.width * c->cfg.height;
+    rtx_ctx::Lane& l0 = c->lane[0];
     // pipelined passes (see rtx_ctx): the estimator E0 without per-launch instrumentation, frames large enough to be cut into path ranges
     const bool eligible = c->pipeline && !(c->cfg.flags & (RTX_FLAG_LEGACY_RR | RTX_FLAG_RESTIR)) &&
-                          !c->timing.stage_timing && !c->trace_stats && (uint64_t)npx * c->cfg.samples_per_pass >= 65536u && lane_buffers(c);
+                          !l0.timing.stage_timing && !c->trace_stats && (uint64_t)npx * c->cfg.samples_per_pass >= 65536u && lane_buffers(c);
     uint32_t done = 0;
     while (done < n_samples) {
         const uint32_t spp = std::min(c->cfg.samples_per_pass, n_samples - done);
-        c->timing.stats = c->trace_stats ? c->d_stats : nullptr;
+        l0.timing.stats = c->trace_stats ? c->d_stats : nullptr;
         // whatever other entry points queued on the caller's stream (camera, instances, uploads, clears) is ordered before the passes of
         // both lanes through ev_state, recorded BEFORE this pass is queued (a lane never waits for the other lane's pass)
         if (c->main_dirty) { RTX_CK(cudaEventRecord(c->ev_state, c->stream)); c->main_dirty = false; }
@@ -791,47 +832,30 @@ extern "C" rtx_status rtx_render_pass(rtx_ctx* c, uint32_t first_sample, uint32_
         const int frame_lane = eligible ? c->pending_lane : -1;       // >= 0: a frame prepared by the fast rtx_set_instances [+ rtx_set_camera]
         if (!(eligible && (c->in_sequence || frame_lane >= 0))) {
             // the first pass after any other call: B.parts path ranges on the caller's stream, accumulation included
-            const SceneData S = scene_data(c);
-            const SceneAS AS = make_as(c);
-            if (c->cam_block_version[0] != c->cam_version) {
-                RTX_CK(cudaMemcpyAsync(c->wb.cam, &c->cam, sizeof c->cam, cudaMemcpyHostToDevice, c->stream));
-                c->cam_block_version[0] = c->cam_version;
-            }
-            if (c->cfg.flags & RTX_FLAG_LEGACY_RR) RTX_CK(wave_render_pass_legacy(c->wb, S, AS, first_sample + done, spp, c->stream, &c->launches, &c->timing));
-            else if (c->cfg.flags & RTX_FLAG_FAST_MATH) RTX_CK(fast::wave_render_pass(c->wb, S, AS, first_sample + done, spp, c->stream, &c->launches, &c->timing));
-            else RTX_CK(wave_render_pass(c->wb, S, AS, first_sample + done, spp, c->stream, &c->launches, &c->timing));
-            RTX_CK(cudaEventRecord(c->ev_acc[0], c->stream));
-            c->last_lane = 0; c->lane_read_set[0] = 0;
+            if ((st = lane_camera(c, l0, c->stream)) != RTX_OK) return st;
+            RTX_CK(run_pass(c, l0, 0, first_sample + done, spp, c->stream, false));
+            RTX_CK(cudaEventRecord(l0.ev_acc, c->stream));
+            c->last_lane = 0; l0.read_set = 0;
         } else {
             // a pass that directly follows another (or a pipelined frame): the other lane, one path range, its accumulation behind the
             // previous pass's
-            const int lane = frame_lane >= 0 ? frame_lane : 1 - c->last_lane;
+            const int i = frame_lane >= 0 ? frame_lane : 1 - c->last_lane;
             const int set = frame_lane >= 0 ? frame_lane : c->cur_set;       // the per-frame state it reads
-            const SceneData S = scene_data(c, set);
-            const SceneAS AS = make_as(c, set);
-            WaveBuffers& B = lane ? c->wb2 : c->wb;
-            PassTiming& T = lane ? c->timing2 : c->timing;
-            const cudaStream_t st_ = c->lane_stream[lane];
+            rtx_ctx::Lane& l = c->lane[i];
+            const cudaStream_t st_ = l.stream;
             RTX_CK(cudaStreamWaitEvent(st_, c->ev_state, 0));
-            RTX_CK(cudaStreamWaitEvent(st_, c->ev_acc[lane], 0));           // the previous pass in these buffers (it may have run on the caller's stream)
-            if (lane) {
-                if (!c->wb.use_graph) B.use_graph = false;
-                T.stage_timing = false; T.stats = nullptr;
-            }
-            if (c->cam_block_version[lane] != c->cam_version) {              // the lane's camera block lags behind the last rtx_set_camera
-                RTX_CK(cudaMemcpyAsync(B.cam, &c->cam, sizeof c->cam, cudaMemcpyHostToDevice, st_));
-                c->cam_block_version[lane] = c->cam_version;
-            }
-            if (c->cfg.flags & RTX_FLAG_FAST_MATH) RTX_CK(fast::wave_render_pass(B, S, AS, first_sample + done, spp, st_, &c->launches, &T, true, 1, true));
-            else RTX_CK(wave_render_pass(B, S, AS, first_sample + done, spp, st_, &c->launches, &T, true, 1, true));
-            RTX_CK(cudaStreamWaitEvent(st_, c->ev_acc[1 - lane], 0));                         // gPermanentData += in call order
+            RTX_CK(cudaStreamWaitEvent(st_, l.ev_acc, 0));          // the previous pass in these buffers (it may have run on the caller's stream)
+            if (!l0.wb.use_graph) l.wb.use_graph = false;           // (a failed capture turns the graphs of both lanes off)
+            if ((st = lane_camera(c, l, st_)) != RTX_OK) return st;
+            RTX_CK(run_pass(c, l, set, first_sample + done, spp, st_, true));
+            RTX_CK(cudaStreamWaitEvent(st_, c->lane[1 - i].ev_acc, 0));                       // gPermanentData += in call order
             if (c->reduce_pending) RTX_CK(cudaStreamWaitEvent(st_, c->ev_reduced, 0));        // a pending multi-GPU reduce still reads it
             if (c->resolve_pending) RTX_CK(cudaStreamWaitEvent(st_, c->ev_resolved, 0));      // ... or the resolve of the previous frame
-            RTX_CK(wave_accumulate(B, npx, spp, st_));
+            RTX_CK(wave_accumulate(l.wb, npx, spp, st_));
             c->launches += 1;
-            RTX_CK(cudaEventRecord(c->ev_acc[lane], st_));
-            RTX_CK(cudaStreamWaitEvent(c->stream, c->ev_acc[lane], 0));     // stream-ordered API: the caller's stream sees the pass as done
-            c->last_lane = lane; c->lane_read_set[lane] = set;
+            RTX_CK(cudaEventRecord(l.ev_acc, st_));
+            RTX_CK(cudaStreamWaitEvent(c->stream, l.ev_acc, 0));    // stream-ordered API: the caller's stream sees the pass as done
+            c->last_lane = i; l.read_set = set;
         }
         c->in_sequence = true; c->pending_lane = -1; c->fset_pending = false;
         done += spp;
@@ -863,11 +887,12 @@ extern "C" rtx_status rtx_render_frame(rtx_ctx* c, uint32_t frame_index) {
     if ((st = ensure_restir(c)) != RTX_OK) return st;
     const SceneData S = scene_data(c);
     const SceneAS AS = make_as(c);
-    c->timing.stats = c->trace_stats ? c->d_stats : nullptr;
-    if (c->wb.wait_before_accumulate) RTX_CK(cudaStreamWaitEvent(c->stream, c->wb.wait_before_accumulate, 0));   // a pending reduce reads gPermanentData
-    RTX_CK(wave_render_pass(c->wb, S, AS, frame_index, 1, c->stream, &c->launches, &c->timing, false));     // RayGen
-    RTX_CK(restir_store_pass1(c->rs, c->wb, S, c->stream, &c->launches));
-    RTX_CK(restir_reuse_passes(c->rs, c->wb, S, AS, frame_index, c->stream, &c->launches));                 // RayGen2, RayGen3
+    rtx_ctx::Lane& l0 = c->lane[0];
+    l0.timing.stats = c->trace_stats ? c->d_stats : nullptr;
+    if (c->reduce_pending) RTX_CK(cudaStreamWaitEvent(c->stream, c->ev_reduced, 0));     // a pending reduce reads gPermanentData
+    RTX_CK(wave_render_pass(l0.wb, S, AS, frame_index, 1, c->stream, &c->launches, &l0.timing, nullptr, false));    // RayGen
+    RTX_CK(restir_store_pass1(c->rs, l0.wb, S, c->stream, &c->launches));
+    RTX_CK(restir_reuse_passes(c->rs, l0.wb, S, AS, frame_index, c->stream, &c->launches));                 // RayGen2, RayGen3
     c->pass_timed = true;
     return RTX_OK;
 }
@@ -895,7 +920,7 @@ extern "C" rtx_status rtx_reset_accum(rtx_ctx* c) {
     RTX_ENTER(c);
     rtx_status st;
     if ((st = ensure_wave(c)) != RTX_OK) return st;
-    RTX_CK(cudaMemsetAsync(c->wb.accum, 0, (size_t)c->cfg.width * c->cfg.height * 16, c->stream));
+    RTX_CK(cudaMemsetAsync(c->d_accum, 0, (size_t)c->cfg.width * c->cfg.height * 16, c->stream));
     return RTX_OK;
 }
 
@@ -911,9 +936,14 @@ extern "C" rtx_status rtx_read_accum(rtx_ctx* c, float* host_out) {
     RTX_ENTER(c);
     rtx_status st;
     if ((st = ensure_wave(c)) != RTX_OK) return st;
-    RTX_CK(cudaMemcpyAsync(host_out, c->wb.accum, (size_t)c->cfg.width * c->cfg.height * 16, cudaMemcpyDeviceToHost, c->stream));
+    RTX_CK(cudaMemcpyAsync(host_out, c->d_accum, (size_t)c->cfg.width * c->cfg.height * 16, cudaMemcpyDeviceToHost, c->stream));
     RTX_CK(cudaStreamSynchronize(c->stream));
     return check_overflow(c);
+}
+
+// gOutput from gPermanentData, or from the buffer rtx_set_resolve_source named
+static cudaError_t resolve(rtx_ctx* c, cudaStream_t s) {
+    return wave_resolve(c->resolve_source ? c->resolve_source : c->d_accum, c->d_output, c->cfg.width * c->cfg.height, s, &c->launches);
 }
 
 extern "C" rtx_status rtx_read_output(rtx_ctx* c, uint8_t* rgba8_out) {
@@ -924,8 +954,8 @@ extern "C" rtx_status rtx_read_output(rtx_ctx* c, uint8_t* rgba8_out) {
     const uint32_t npx = c->cfg.width * c->cfg.height;
     if (c->copy_pending) { RTX_CK(cudaEventSynchronize(c->ev_copied)); c->copy_pending = false; }
     if (c->comm && c->ev_reduced) RTX_CK(cudaStreamWaitEvent(c->stream, c->ev_reduced, 0));      // the reduced buffer must be complete
-    RTX_CK(wave_resolve(c->wb, npx, c->stream, &c->launches));
-    RTX_CK(cudaMemcpyAsync(rgba8_out, c->wb.output, (size_t)npx * 4, cudaMemcpyDeviceToHost, c->stream));
+    RTX_CK(resolve(c, c->stream));
+    RTX_CK(cudaMemcpyAsync(rgba8_out, c->d_output, (size_t)npx * 4, cudaMemcpyDeviceToHost, c->stream));
     return check_overflow(c);       // synchronises the stream
 }
 
@@ -952,17 +982,17 @@ extern "C" rtx_status rtx_read_output_async(rtx_ctx* c, uint8_t* rgba8_out) {
     if ((st = ensure_wave(c)) != RTX_OK) return st;
     if ((st = ensure_side_stream(c)) != RTX_OK) return st;
     const uint32_t npx = c->cfg.width * c->cfg.height;
-    if (c->comm && c->comm_rank == 0 && c->wb.resolve_source == c->d_total) {
+    if (c->comm && c->comm_rank == 0 && c->resolve_source == c->d_total) {
         // side stream order: reduce(k) -> resolve(k) -> copy(k) -> reduce(k+1) ...: nothing else touches d_total or gOutput
-        RTX_CK(wave_resolve(c->wb, npx, c->copy_stream, &c->launches));
+        RTX_CK(resolve(c, c->copy_stream));
     } else {
         if (c->copy_pending) RTX_CK(cudaStreamWaitEvent(c->stream, c->ev_copied, 0));      // gOutput is rewritten by the resolve below
-        RTX_CK(wave_resolve(c->wb, npx, c->stream, &c->launches));
+        RTX_CK(resolve(c, c->stream));
         RTX_CK(cudaEventRecord(c->ev_resolved, c->stream));
         RTX_CK(cudaStreamWaitEvent(c->copy_stream, c->ev_resolved, 0));
         c->resolve_pending = true;
     }
-    RTX_CK(cudaMemcpyAsync(rgba8_out, c->wb.output, (size_t)npx * 4, cudaMemcpyDeviceToHost, c->copy_stream));
+    RTX_CK(cudaMemcpyAsync(rgba8_out, c->d_output, (size_t)npx * 4, cudaMemcpyDeviceToHost, c->copy_stream));
     RTX_CK(cudaMemcpyAsync(c->h_overflow, c->d_overflow, sizeof(unsigned int), cudaMemcpyDeviceToHost, c->copy_stream));   // for rtx_wait_output
     RTX_CK(cudaEventRecord(c->ev_copied, c->copy_stream));
     c->copy_pending = true;
@@ -976,7 +1006,7 @@ extern "C" rtx_status rtx_set_resolve_source(rtx_ctx* c, const void* d_accum_flo
     RTX_ENTER(c);
     rtx_status st;
     if ((st = ensure_wave(c)) != RTX_OK) return st;
-    c->wb.resolve_source = (const float4*)d_accum_float4;
+    c->resolve_source = (const float4*)d_accum_float4;
     return RTX_OK;
 }
 
@@ -1000,7 +1030,7 @@ extern "C" rtx_status rtx_accum_device_ptr(rtx_ctx* c, void** out) {
     RTX_ENTER(c);
     rtx_status st;
     if ((st = ensure_wave(c)) != RTX_OK) return st;
-    *out = c->wb.accum;
+    *out = c->d_accum;
     return RTX_OK;
 }
 
@@ -1049,8 +1079,8 @@ static rtx_status trace_device_impl(rtx_ctx* c, const void* d_rays, uint32_t n, 
     const unsigned grid = (n + 255) / 256;
     k_split_rays<<<grid, 256, 0, c->stream>>>((const float4*)d_rays, n, c->d_trace_o, c->d_trace_d);
     // the cursor word of part 0 of the wavefront buffers
-    if (!c->wb_ready) { if ((st = ensure_wave(c)) != RTX_OK) return st; }
-    RTX_CK(launch_trace(make_as(c), c->d_trace_o, c->d_trace_d, nullptr, n, c->wb.cursor, c->d_trace_ha, c->d_trace_hi, any_hit != 0,
+    if (!c->lane[0].ready) { if ((st = ensure_wave(c)) != RTX_OK) return st; }
+    RTX_CK(launch_trace(make_as(c), c->d_trace_o, c->d_trace_d, nullptr, n, c->lane[0].wb.cursor, c->d_trace_ha, c->d_trace_hi, any_hit != 0,
                         stats ? c->d_stats : nullptr, c->stream));
     k_pack_hits<<<grid, 256, 0, c->stream>>>(c->d_trace_ha, c->d_trace_hi, n, any_hit, c->d_trace_d, (rtx_hit*)d_hits);
     c->launches += 3;
@@ -1140,7 +1170,7 @@ extern "C" rtx_status rtx_comm_destroy(rtx_ctx* c) {
     if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
     nccl().CommDestroy(c->comm);
     c->comm = nullptr; c->comm_world = 1; c->comm_rank = 0;
-    if (c->wb_ready) { if (c->wb.resolve_source == c->d_total) c->wb.resolve_source = nullptr; c->wb.wait_before_accumulate = nullptr; }
+    if (c->resolve_source == c->d_total) c->resolve_source = nullptr;
     c->reduce_pending = false;
     if (c->d_total) { cudaFree(c->d_total); c->d_total = nullptr; }
     if (c->ev_pass) { cudaEventDestroy(c->ev_pass); c->ev_pass = nullptr; }
@@ -1169,7 +1199,7 @@ extern "C" rtx_status rtx_comm_init(rtx_ctx* c, const void* unique_id128, int ra
         const size_t bytes = (size_t)c->cfg.width * c->cfg.height * 16;
         RTX_CK(cudaMalloc((void**)&c->d_total, bytes));
         RTX_CK(cudaMemsetAsync(c->d_total, 0, bytes, c->stream));
-        c->wb.resolve_source = c->d_total;          // "rank 0 then runs F20's divide + sRGB" on the sum
+        c->resolve_source = c->d_total;             // "rank 0 then runs F20's divide + sRGB" on the sum
     }
     return RTX_OK;
 }
@@ -1185,11 +1215,10 @@ extern "C" rtx_status rtx_reduce_accum(rtx_ctx* c) {
     RTX_CK(cudaEventRecord(c->ev_pass, c->stream));
     RTX_CK(cudaStreamWaitEvent(c->copy_stream, c->ev_pass, 0));
     const size_t count = (size_t)c->cfg.width * c->cfg.height * 4;
-    const int r = nccl().Reduce(c->wb.accum, c->comm_rank == 0 ? (void*)c->d_total : (void*)c->wb.accum, count, /*ncclFloat32*/ 7, /*ncclSum*/ 0, 0,
+    const int r = nccl().Reduce(c->d_accum, c->comm_rank == 0 ? (void*)c->d_total : (void*)c->d_accum, count, /*ncclFloat32*/ 7, /*ncclSum*/ 0, 0,
                                 c->comm, c->copy_stream);
     if (r != 0) return nccl_fail("ncclReduce", r);
     RTX_CK(cudaEventRecord(c->ev_reduced, c->copy_stream));
-    c->wb.wait_before_accumulate = c->ev_reduced;
     c->reduce_pending = true;
     return RTX_OK;
 }
@@ -1209,14 +1238,11 @@ extern "C" rtx_status rtx_get_counters(rtx_ctx* c, rtx_counters* out) {
     RTX_ENTER(c);
     memset(out, 0, sizeof *out);
     RTX_CK(cudaStreamSynchronize(c->stream));
-    if (c->wb_ready) {
+    for (auto& l : c->lane) {
+        if (!l.ready) continue;
         unsigned long long h[8];
-        RTX_CK(cudaMemcpy(h, c->wb.ray_counters, sizeof h, cudaMemcpyDeviceToHost));
-        out->closest_rays = h[0]; out->shadow_rays = h[1]; out->paths = h[2];
-        if (c->wb2_ready) {
-            RTX_CK(cudaMemcpy(h, c->wb2.ray_counters, sizeof h, cudaMemcpyDeviceToHost));
-            out->closest_rays += h[0]; out->shadow_rays += h[1]; out->paths += h[2];
-        }
+        RTX_CK(cudaMemcpy(h, l.wb.ray_counters, sizeof h, cudaMemcpyDeviceToHost));
+        out->closest_rays += h[0]; out->shadow_rays += h[1]; out->paths += h[2];
     }
     TraceStats ts;
     RTX_CK(cudaMemcpy(&ts, c->d_stats, sizeof ts, cudaMemcpyDeviceToHost));
@@ -1230,8 +1256,7 @@ extern "C" rtx_status rtx_reset_counters(rtx_ctx* c) {
     if (!c) return fail(RTX_ERR_ARG, "null context");
     RTX_ENTER(c);
     RTX_CK(cudaStreamSynchronize(c->stream));
-    if (c->wb_ready) RTX_CK(cudaMemset(c->wb.ray_counters, 0, 64));
-    if (c->wb2_ready) RTX_CK(cudaMemset(c->wb2.ray_counters, 0, 64));
+    for (auto& l : c->lane) if (l.ready) RTX_CK(cudaMemset(l.wb.ray_counters, 0, 64));
     RTX_CK(cudaMemset(c->d_stats, 0, sizeof(TraceStats)));
     c->launches = 0;
     return RTX_OK;
@@ -1241,18 +1266,14 @@ static rtx_status stage_ms(rtx_ctx* c, float* by_kind, float* total) {
     if (!c->pass_timed) return fail(RTX_ERR_STATE, "rtx_last_pass_ms: no pass rendered yet");
     RTX_CK(cudaSetDevice(c->cfg.device));
     for (int k = 0; k < SK_COUNT; k++) by_kind[k] = 0.0f;
-    if (c->last_lane == 1) {        // the last pass ran on the second lane (pipelined passes carry no per-launch events)
-        RTX_CK(cudaEventSynchronize(c->timing2.ev[1]));
-        RTX_CK(cudaEventElapsedTime(total, c->timing2.ev[0], c->timing2.ev[1]));
-        return RTX_OK;
-    }
-    RTX_CK(cudaEventSynchronize(c->timing.ev[1]));
-    RTX_CK(cudaEventElapsedTime(total, c->timing.ev[0], c->timing.ev[1]));
-    for (int i = 0; i < c->timing.n_marks; i++) {
+    const PassTiming& T = c->lane[c->last_lane].timing;       // (a pipelined pass carries no per-launch events: n_marks == 0)
+    RTX_CK(cudaEventSynchronize(T.ev[1]));
+    RTX_CK(cudaEventElapsedTime(total, T.ev[0], T.ev[1]));
+    for (int i = 0; i < T.n_marks; i++) {
         float d = 0.0f;
-        cudaEvent_t next = (i + 1 < c->timing.n_marks) ? c->timing.ev[3 + i] : c->timing.ev[1];
-        RTX_CK(cudaEventElapsedTime(&d, c->timing.ev[2 + i], next));
-        by_kind[c->timing.kind[i]] += d;
+        cudaEvent_t next = (i + 1 < T.n_marks) ? T.ev[3 + i] : T.ev[1];
+        RTX_CK(cudaEventElapsedTime(&d, T.ev[2 + i], next));
+        by_kind[T.kind[i]] += d;
     }
     return RTX_OK;
 }
@@ -1281,13 +1302,13 @@ extern "C" rtx_status rtx_set_option(rtx_ctx* c, uint32_t option, uint32_t value
     if (!c) return fail(RTX_ERR_ARG, "null context");
     RTX_ENTER(c);
     if (option == RTX_OPT_TRACE_STATS) c->trace_stats = value != 0;
-    else if (option == RTX_OPT_STAGE_TIMING) c->timing.stage_timing = value != 0;
+    else if (option == RTX_OPT_STAGE_TIMING) c->lane[0].timing.stage_timing = value != 0;
     else if (option == RTX_OPT_TLAS_REBUILD) c->force_tlas_rebuild = value != 0;
     else if (option == RTX_OPT_PASS_PARTS) {
         if (value < 1u || value > (uint32_t)WAVE_MAX_PARTS) return fail(RTX_ERR_ARG, "rtx_set_option: RTX_OPT_PASS_PARTS must be 1..4");
-        c->wb.parts = (int)value;
+        c->lane[0].wb.parts = (int)value;
     }
-    else if (option == RTX_OPT_PASS_GRAPH) { c->wb.use_graph = value != 0; c->wb2.use_graph = value != 0; }
+    else if (option == RTX_OPT_PASS_GRAPH) { for (auto& l : c->lane) l.wb.use_graph = value != 0; }
     else if (option == RTX_OPT_PASS_PIPELINE) c->pipeline = value != 0;
     else if (option == RTX_OPT_FRAME_PIPELINE) c->frame_pipeline = value != 0;
     else return fail(RTX_ERR_ARG, "rtx_set_option: unknown option");
@@ -1304,10 +1325,10 @@ extern "C" rtx_status rtx_selftest_dmath(rtx_ctx* c, uint64_t* out, uint32_t n_o
 }
 
 extern "C" rtx_status rtx_debug_pixel(rtx_ctx* c, uint32_t x, uint32_t y, float* out64) {
-    if (!c || !out64 || !c->wb_ready) return fail(RTX_ERR_ARG, "rtx_debug_pixel: bad argument");
+    if (!c || !out64 || !c->lane[0].ready) return fail(RTX_ERR_ARG, "rtx_debug_pixel: bad argument");
     if (x >= c->cfg.width || y >= c->cfg.height) return fail(RTX_ERR_ARG, "rtx_debug_pixel: pixel out of range");
     RTX_ENTER(c);
     SceneData S; memset(&S, 0, sizeof S); S.width = c->cfg.width; S.height = c->cfg.height;
-    RTX_CK(wave_debug_pixel(c->wb, S, x, y, c->stream, out64));
+    RTX_CK(wave_debug_pixel(c->lane[0].wb, S, x, y, c->stream, out64));
     return RTX_OK;
 }

@@ -1,8 +1,10 @@
-// wave_dev.cuh — device helpers shared by the wavefront stages (wavefront.cu) and the ReSTIR reuse passes (restir.cu).
+// wave_dev.cuh — device helpers shared by the wavefront stages (wavefront.cu, wave_common.cu) and the ReSTIR reuse passes (restir.cu).
 #pragma once
 #include "wavefront.h"
 
 namespace rtx {
+
+#define WF_BLOCK 128        // CTA size of the wavefront's per-path and per-pixel kernels
 
 struct StateView {
     float4* base; uint32_t n;

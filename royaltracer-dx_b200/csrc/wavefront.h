@@ -43,6 +43,7 @@ struct RayQueue {
 };
 
 #define WAVE_MAX_PARTS 4
+// One lane's pass buffers (api.cu: a context has two).  gPermanentData and gOutput belong to the context.
 struct WaveBuffers {
     uint32_t n_paths = 0;
     int parts = 2;                     // path ranges of a pass that run concurrently on separate streams (wave_render_pass)
@@ -59,20 +60,18 @@ struct WaveBuffers {
     uint32_t* counts = nullptr;        // 4 queue counters + scratch
     unsigned int* cursor = nullptr;    // 4 words per part (launch_trace)
     unsigned long long* ray_counters = nullptr;   // [0] closest, [1] shadow, [2] paths
-    const float4* resolve_source = nullptr;   // rtx_set_resolve_source: an external accumulation buffer (the multi-GPU sum) to resolve instead
     uint32_t* first_sample = nullptr;  // device word: the sample index of the pass being rendered (k_generate reads it)
     // CUDA graph of a pass (wavefront.cu wave_render_pass): replayed while the configuration (graph_key) stays what was captured
     struct GraphSlot { cudaGraphExec_t exec = nullptr; uint64_t launches = 0, last_used = 0; unsigned char key[512] = {}; };
     bool use_graph = true, have_last_key = false; GraphSlot graphs[4]; uint64_t graph_clock = 0;
     unsigned char last_key[512] = {};
-    cudaEvent_t wait_before_accumulate = nullptr;   // multi-GPU: the pending reduce of gPermanentData (k_accumulate rewrites it)
-    float4* accum = nullptr;           // gPermanentData
-    uint8_t* output = nullptr;         // gOutput slice 0
+    float4* accum = nullptr;           // gPermanentData, borrowed from the context (wave_free leaves it alone)
     rtx_camera_params* cam = nullptr;  // b0 (device copy)
     float* debug = nullptr;            // 64 floats
 };
 
-cudaError_t wave_alloc(WaveBuffers* B, uint32_t width, uint32_t height, uint32_t spp);
+// the pass buffers for spp samples of a width x height frame, accumulating into `accum`
+cudaError_t wave_alloc(WaveBuffers* B, float4* accum, uint32_t width, uint32_t height, uint32_t spp);
 void wave_free(WaveBuffers* B);
 
 #define WAVE_MAX_EVENTS 96
@@ -87,25 +86,25 @@ struct PassTiming {
 };
 
 // One DispatchRays-equivalent: samples [first_sample, first_sample + spp) of every pixel.
+// reduce: null, or the event of a multi-GPU reduce that may still read gPermanentData (the final k_accumulate waits for it).
 // parts_override > 0: that many path ranges instead of B.parts.  defer_accumulate: everything but the final k_accumulate (the caller
 // launches wave_accumulate itself, behind whatever has to touch gPermanentData first: api.cu pipelines consecutive passes that way).
 cudaError_t wave_render_pass(WaveBuffers& B, const SceneData& S, const SceneAS& AS, uint32_t first_sample, uint32_t spp,
-                             cudaStream_t stream, uint64_t* launches, PassTiming* timing, bool accumulate = true, int parts_override = 0,
-                             bool defer_accumulate = false);
+                             cudaStream_t stream, uint64_t* launches, PassTiming* timing, cudaEvent_t reduce, bool accumulate = true,
+                             int parts_override = 0, bool defer_accumulate = false);
 // the same stage sequence built with fast math (wavefront.cu compiled with -DRTX_FAST_MATH): RTX_FLAG_FAST_MATH
 namespace fast {
 cudaError_t wave_render_pass(WaveBuffers& B, const SceneData& S, const SceneAS& AS, uint32_t first_sample, uint32_t spp,
-                             cudaStream_t stream, uint64_t* launches, PassTiming* timing, bool accumulate = true, int parts_override = 0,
-                             bool defer_accumulate = false);
+                             cudaStream_t stream, uint64_t* launches, PassTiming* timing, cudaEvent_t reduce, bool accumulate = true,
+                             int parts_override = 0, bool defer_accumulate = false);
 }
-// a second set of pass buffers that shares gPermanentData and gOutput with `B` (pipelined passes, api.cu)
-cudaError_t wave_alloc_lane(WaveBuffers* L, const WaveBuffers& B, uint32_t width, uint32_t height, uint32_t spp);
-void wave_free_lane(WaveBuffers* L);
 // The reference's legacy estimator (include/RayGen.hlsl + include/Hit.hlsl) as a wavefront: legacy.cu.  S.bounces caps the path length.
 cudaError_t wave_render_pass_legacy(WaveBuffers& B, const SceneData& S, const SceneAS& AS, uint32_t first_sample, uint32_t spp,
                                     cudaStream_t stream, uint64_t* launches, PassTiming* timing);
+// wave_alloc / wave_free and the functions below are compiled once (wave_common.cu), whichever build rendered the pass.
 cudaError_t wave_accumulate(WaveBuffers& B, uint32_t npx, uint32_t spp, cudaStream_t stream);   // k_accumulate over SP_RESULT
-cudaError_t wave_resolve(WaveBuffers& B, uint32_t n_pixels, cudaStream_t stream, uint64_t* launches);
+// gOutput (RGBA8) of the accumulation buffer `accum`
+cudaError_t wave_resolve(const float4* accum, uint8_t* output, uint32_t n_pixels, cudaStream_t stream, uint64_t* launches);
 cudaError_t wave_selftest_dmath(cudaStream_t stream, unsigned long long* host_out, uint32_t n_out);
 cudaError_t wave_debug_pixel(WaveBuffers& B, const SceneData& S, uint32_t x, uint32_t y, cudaStream_t stream, float* host_out64);
 

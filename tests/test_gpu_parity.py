@@ -696,6 +696,47 @@ def test_pipelined_passes_are_bit_identical(rtdx, orc):
     ctx.close()
 
 
+def test_fast_math_pipelined_passes_accumulate_like_unpipelined_ones(rtdx):
+    """RTX_FLAG_FAST_MATH with RTX_OPT_PASS_PIPELINE on and off: a run of passes leaves the same accumulation bit for bit.  The passes
+    on the caller's stream and those on the two lanes add their samples to gPermanentData with one and the same k_accumulate."""
+    sc = rtdx.scenes.mesh_room(n=16)
+    W, H, bounces, n_samples = 384, 192, 3, 7
+    ctx, _ = _upload(rtdx, sc, W, H, bounces=bounces, flags=rtdx.FLAG_FAST_MATH)
+    accs = []
+    for pipeline in (1, 0):
+        ctx.set_option(rtdx.OPT_PASS_PIPELINE, pipeline)
+        ctx.reset_accum()
+        for s in range(n_samples):
+            ctx.render_pass(s, 1)
+        ctx.synchronize()
+        accs.append(ctx.read_accum())
+    assert (accs[0][..., 3] == n_samples).all()
+    assert np.array_equal(bits(accs[0]), bits(accs[1]))
+    ctx.close()
+
+
+def test_last_pass_timing_after_pipelined_and_stage_timed_passes(rtdx):
+    """rtx_last_pass_ms / rtx_last_pass_stage_ms.  After a pipelined sequence, whose last pass ran on either lane and carries no
+    per-launch events, the pass total is positive and every stage is 0.  With RTX_OPT_STAGE_TIMING the stages are non-negative, the
+    closest-hit launches take time, and the stages add up to no more than the pass total."""
+    sc = rtdx.scenes.mesh_room(n=16)
+    ctx, _ = _upload(rtdx, sc, 384, 192, bounces=3)
+    for first, n in ((0, 2), (2, 1)):                   # the sequence goes on across rtx_synchronize: its last pass on lane 1, then lane 0
+        for s in range(first, first + n):
+            ctx.render_pass(s, 1)
+        ctx.synchronize()
+        stages, total = ctx.last_pass_stage_ms()
+        assert total > 0 and all(v == 0.0 for v in stages.values()), (first, stages, total)
+        assert ctx.last_pass_ms() == (0.0, total)
+    ctx.set_option(rtdx.OPT_STAGE_TIMING, 1)
+    ctx.render_pass(3, 1); ctx.synchronize()
+    stages, total = ctx.last_pass_stage_ms()
+    assert all(v >= 0.0 for v in stages.values()) and stages["closest"] > 0, stages
+    assert sum(stages.values()) <= total + 1e-4, (stages, total)
+    assert ctx.last_pass_ms() == (stages["closest"], total)
+    ctx.close()
+
+
 def test_pipelined_frames_are_bit_identical(rtdx, orc):
     """RTX_OPT_FRAME_PIPELINE: a per-frame loop in the reference's order (rtx_set_instances with a moving instance, rtx_set_camera,
     rtx_render_pass, rtx_read_output_async with one frame in flight) on a one-node TLAS keeps two sets of per-frame state and overlaps
